@@ -53,6 +53,28 @@ WORKLOADS = {
 }
 METRIC = "PartialFC CosFace fwd+bwd samples/s"
 S, M = 64.0, 0.4
+# --dump-outputs keeps the files small enough to compare two builds (64 MB at most): a fixed sample of the outputs that are
+# too large to store whole -- rows of the class-shard gradient (split over the ranks), elements of the averaged model (c5)
+DUMP_ROWS = 8192
+DUMP_ELEMS = 4 << 20
+
+
+def sample_index(n, k, seed=0):
+    """Sorted indices of a fixed, seeded sample of k of 0..n-1 (all of them when n <= k), as an int64 tensor."""
+    import numpy as np
+    import torch
+    if n <= k:
+        return torch.arange(n)
+    return torch.from_numpy(np.sort(np.random.default_rng(seed).choice(n, k, replace=False)))
+
+
+def dump_outputs(path, arrays):
+    """Each tensor of ``arrays`` (name -> tensor) as path/<name>.npy: float32, float64 for integer data."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(path, name + ".npy"), (t.float() if t.is_floating_point() else t.double()).numpy())
 
 
 def load_peaks():
@@ -222,6 +244,7 @@ def run_fedavg(args):
     value = algorithmic GB/s ((K+1) * N * 4 bytes per call) of the public ``FedPavg`` call with the clients resident in HBM as
     ``FlatStateDict``s (one flat buffer per client, ``fedfr_b200.flatten_state_dict``); the plain dict-of-477-tensors call is
     timed beside it.  Clients are sharded over the ranks (K/W each) and the partial sums meet in one all-reduce."""
+    import numpy as np
     import torch
     import torch.distributed as dist
     import __graft_entry__ as G
@@ -279,9 +302,24 @@ def run_fedavg(args):
     if sampler:
         sampler.start()
     from fedfr_b200 import _native as N
+    last = [None]
+
+    def call_flats():
+        last[0] = call(flats)
+
     l0 = N.lib.pfc_launch_count()
-    ms = timed(lambda: call(flats), args.steps)
+    ms = timed(call_flats, args.steps)
     launches = N.lib.pfc_launch_count() - l0
+    if args.dump_outputs and rank == 0:          # the averaged model is the same on every rank
+        # a sample of the model's tensors laid end to end (key order), gathered tensor by tensor: no copy of the whole model
+        vals = list(last[0].values())
+        starts = np.cumsum([0] + [v.numel() for v in vals])
+        idx = sample_index(int(starts[-1]), DUMP_ELEMS)
+        cut = np.searchsorted(idx.numpy(), starts)
+        picked = [v.reshape(-1)[(idx[a:b] - int(s)).to(dev)] for v, s, a, b in zip(vals, starts, cut[:-1], cut[1:]) if b > a]
+        dump_outputs(args.dump_outputs, {"fedpavg_sample_index": idx, "fedpavg_sample": torch.cat(picked)})
+        del vals, picked
+    last[0] = None
     # the C-ABI call alone (table upload + the one kernel), re-launched from the tables the last call staged
     from fedfr_b200 import fedavg as FA
     torch.cuda.synchronize()
@@ -466,9 +504,11 @@ def run_ours(args):
     feats_h = feats.cpu().pin_memory()
     label_h = label.cpu().pin_memory()
 
+    last = [None]
+
     def step_resident():
         head.sub_weight.grad = None                      # what optimizer.zero_grad(set_to_none=True) leaves behind
-        return head.forward_backward(label, feats, opt)
+        last[0] = head.forward_backward(label, feats, opt)
 
     xg_h = torch.empty((B, E), dtype=torch.float32).pin_memory()
     loss_h = torch.empty((), dtype=torch.float32).pin_memory()
@@ -513,6 +553,16 @@ def run_ours(args):
     launches = N.lib.pfc_launch_count() - launches0
     clocks = sampler.stop() if sampler else None
     ms_step = ms_total / args.steps
+    if args.dump_outputs:                                # what the caller received from the last timed step
+        x_grad, loss = last[0]
+        grad = head.sub_weight.grad
+        rows = sample_index(grad.shape[0], DUMP_ROWS // world)
+        out = {"x_grad": x_grad, "loss": loss, "sub_weight_grad_rows": rows, "sub_weight_grad": grad[rows.to(dev)]}
+        if head.index is not None:                       # the sampled classes (sample_rate < 1)
+            out["index"] = head.index
+        dump_outputs(args.dump_outputs, {(n + f"_rank{rank}" if world > 1 else n): t for n, t in out.items()})
+        del x_grad, loss, grad, out
+    last[0] = None
 
     for _ in range(2):
         step_e2e()
@@ -747,7 +797,14 @@ def main():
     ap.add_argument("--dw4", type=int, default=-1, help="1/0: 4-CTA-cluster dw kernel (E = 512)")
     ap.add_argument("--prob-split", default="", help="stored-probability backward: 'dx_sms[,dw_rate[,sweep_lead]]' (SM budget of the dx kernel, dx/dw pacing)")
     ap.add_argument("--chunk-mb", type=int, default=0, help="bf16 G scratch per backward chunk in MiB (0 = library default)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step returned to DIR/<name>.npy (float32, integer data as float64; a fixed "
+                         "sample of the large outputs, 64 MB at most) to compare two builds on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     _quiet_stdout()
     if args.impl == "reference":
         run_reference(args)

@@ -1,9 +1,13 @@
-"""bench.py contract pieces that run without a GPU: the reference arm prints exactly one JSON line on stdout (library
-chatter goes to stderr), with the keys the driver reads; ranks other than 0 stay silent."""
+"""bench.py contract pieces: without a GPU, the reference arm prints exactly one JSON line on stdout (library chatter goes
+to stderr) with the keys a harness reads, and ranks other than 0 stay silent; on the GPU, --dump-outputs writes the last
+timed step's outputs."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -38,3 +42,19 @@ def test_reference_arm_prints_one_json_line():
 def test_reference_arm_other_ranks_are_silent():
     r = _run(dict(TORCHRUN_ENV, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1"))
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_last_timed_step(tmp_path):
+    """--dump-outputs: x_grad, the loss and a fixed sample of sub_weight.grad rows of the last timed step, as float .npy files."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--workload", "c2", "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    out = {f[:-len(".npy")]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert sorted(out) == ["loss", "sub_weight_grad", "sub_weight_grad_rows", "x_grad"]
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in out.values())
+    assert sum(os.path.getsize(tmp_path / f) for f in os.listdir(tmp_path)) <= 64 << 20
+    rows = out["sub_weight_grad_rows"]
+    assert out["x_grad"].shape == (512, 512) and out["sub_weight_grad"].shape == (len(rows), 512) and len(rows) == 8192
+    assert np.all(np.diff(rows) > 0) and rows[0] >= 0 and rows[-1] < 100_000 and float(out["loss"]) > 0

@@ -645,7 +645,8 @@ def test_emulated_kernels_under_address_sanitizer():
     if not os.path.isabs(asan) or not os.path.exists(asan):
         pytest.skip("libasan not available")
     env = dict(os.environ, LD_PRELOAD=asan, EMU_ASAN="1", EMU_SCHEDULE="reverse",      # and the opposite thread/block order
-               ASAN_OPTIONS="detect_leaks=0:detect_stack_use_after_return=0")
+               ASAN_OPTIONS="detect_leaks=0:detect_stack_use_after_return=0",
+               CUDA_VISIBLE_DEVICES="")      # the emulation needs no device: keep the GPU driver out of the instrumented process
     r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-x", "-q", "-p", "no:cacheprovider",
                         "-k", "not property and not sgd_step and not stats_abi and not check_mode"],     # time budget: the sweeps and
                        # the slowest B200-validated kernels stay in the plain pass only

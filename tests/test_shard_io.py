@@ -1,8 +1,8 @@
 """Shard I/O of PartialFC (partial_fc.py:38-60 resume, :71-87 save_params / save_FC / update_FC / update_from_tensor):
 file names, file contents, resume fall-backs and the sub_weight aliasing, on CPU through the host-logic provider
-(tests/oracle_ops.py) and on the GPU through the real kernels.  Where /root/reference exists the files are exchanged
-with the unmodified reference class in both directions."""
+(tests/oracle_ops.py) and on the GPU through the real kernels."""
 import os
+import shutil
 import sys
 
 import pytest
@@ -10,7 +10,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
-REF = "/root/reference"
+GOLDEN_FILES = ("rank:0_softmax_weight.pt", "rank:0_softmax_weight_mom.pt", "FC_rank_0.pth")
 
 
 @pytest.fixture(scope="module")
@@ -115,30 +115,23 @@ def test_update_from_tensor(pkg, tmp_path):
     assert float((x_grad - ref.x_grad[0]).abs().max()) < 1e-5
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "partial_fc.py")), reason="reference checkout not present")
 def test_files_interchange_with_reference_class(pkg, tmp_path):
-    """The unmodified reference methods write the files; this package resumes from them, and the other way round."""
-    sys.path.insert(0, REF)
-    import partial_fc as ref_mod
-    r = ref_mod.PartialFC.__new__(ref_mod.PartialFC)              # its ctor hard-codes CUDA (partial_fc.py:27,61,69)
-    torch.nn.Module.__init__(r)
-    g = torch.Generator().manual_seed(4)
-    r.prefix, r.rank, r.local_rank = str(tmp_path), 0, 0
-    r.weight = torch.randn(300, 64, generator=g) * 0.01
-    r.weight_mom = torch.randn(300, 64, generator=g) * 0.001
-    r.weight_name = os.path.join(r.prefix, "rank:{}_softmax_weight.pt".format(r.rank))
-    r.weight_mom_name = os.path.join(r.prefix, "rank:{}_softmax_weight_mom.pt".format(r.rank))
-    r.save_params()                                               # partial_fc.py:71-73
-    r.save_FC()                                                   # partial_fc.py:75-76
+    """The files the unmodified reference methods wrote (save_params / save_FC, tests/golden/make_golden_shard_io.py): this
+    package resumes from them and loads them with update_FC, and the files it writes load back with plain torch.load."""
+    for f in GOLDEN_FILES:
+        shutil.copyfile(os.path.join(HERE, "golden", "shard_io", f), os.path.join(str(tmp_path), f))
+    g = torch.Generator().manual_seed(4)                            # the tensors the reference saved
+    w = torch.randn(300, 64, generator=g) * 0.01
+    mom = torch.randn(300, 64, generator=g) * 0.001
     h = _head(pkg, tmp_path, resume=True)
-    assert h.weight_name == r.weight_name and h.weight_mom_name == r.weight_mom_name
-    assert torch.equal(h.weight, r.weight) and torch.equal(h.weight_mom, r.weight_mom)
+    assert h.weight_name == os.path.join(str(tmp_path), GOLDEN_FILES[0]) and h.weight_mom_name == os.path.join(str(tmp_path), GOLDEN_FILES[1])
+    assert torch.equal(h.weight, w) and torch.equal(h.weight_mom, mom)
     h2 = _head(pkg, tmp_path)
     h2.update_FC()
-    assert torch.equal(h2.weight, r.weight)
+    assert torch.equal(h2.weight, w)
     _train_one_step(h)
-    h.save_params()                                               # ... and back: what partial_fc.py:43,50 would load
-    assert torch.equal(torch.load(r.weight_name), h.weight) and torch.equal(torch.load(r.weight_mom_name), h.weight_mom)
+    h.save_params()                                                 # ... and back: what partial_fc.py:43,50 would load
+    assert torch.equal(torch.load(h.weight_name), h.weight) and torch.equal(torch.load(h.weight_mom_name), h.weight_mom)
 
 
 @pytest.mark.gpu
@@ -163,28 +156,3 @@ def test_gpu_checkpoint_roundtrip_and_loaders(pkg, tmp_path, sr):
         # which shard was used, not kernel numerics (those are test_gpu_parity's job): a stale shard is off by O(1)
         assert abs(float(loss) - float(ref.loss)) < 5e-2 * abs(float(ref.loss))
         assert float((x_grad.cpu() - ref.x_grad[0]).norm() / ref.x_grad[0].norm()) < 5e-2
-
-
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "utils", "utils_callbacks.py")), reason="reference checkout not present")
-def test_reference_checkpoint_callback_drives_this_class(pkg, tmp_path):
-    """utils/utils_callbacks.py:115-124 (CallBackModelCheckpoint, the reference's only consumer of PartialFC.save_params) run
-    unmodified with this package's PartialFC in place of the reference's."""
-    import types
-    for name in ("easydict", "mxnet", "prettytable"):                  # import-time dependencies of the reference, absent here
-        sys.modules.setdefault(name, types.ModuleType(name))
-    sys.modules["easydict"].EasyDict = getattr(sys.modules["easydict"], "EasyDict", dict)
-    for sub in ("ndarray", "recordio", "image"):
-        m = sys.modules.setdefault("mxnet." + sub, types.ModuleType("mxnet." + sub))
-        setattr(sys.modules["mxnet"], sub, m)
-    sys.modules["prettytable"].PrettyTable = getattr(sys.modules["prettytable"], "PrettyTable", object)
-    sys.path.insert(0, REF)
-    from utils.utils_callbacks import CallBackModelCheckpoint
-    head = _head(pkg, tmp_path)
-    _train_one_step(head)
-    backbone = types.SimpleNamespace(module=torch.nn.Linear(4, 4))
-    cb = CallBackModelCheckpoint(rank=0, output=str(tmp_path))
-    cb(0, backbone, head)
-    assert os.listdir(tmp_path) == []                                   # global_step == 0: nothing is written (:121,123)
-    cb(7, backbone, head)
-    assert sorted(os.listdir(tmp_path)) == ["backbone.pth", "rank:0_softmax_weight.pt", "rank:0_softmax_weight_mom.pt"]
-    assert torch.equal(torch.load(head.weight_name), head.weight) and torch.equal(torch.load(head.weight_mom_name), head.weight_mom)
