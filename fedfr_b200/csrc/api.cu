@@ -212,7 +212,7 @@ int pfc_set_prefetch(int logits, int dx_distance, int dw) {   /* TMA L2 prefetch
   return 0;
 }
 
-int pfc_set_dx_pair(int on) {   /* 1 = CTA-pair dx kernel when Bt % 512 == 0 (default), 0 = single-CTA kernel */
+int pfc_set_dx_pair(int on) {   /* 1 = CTA-pair dx kernel when the row blocks come in fours (ceil(Bt / 128) % 4 == 0), E >= 256 and the pair logits kernels are on (default), 0 = single-CTA kernel */
   tc_set_dx_pair(on);
   return 0;
 }

@@ -1996,7 +1996,7 @@ struct BwdPlan {
   bool pipelined;
   int sm_g, sm_dx, sm_dw;   // SMs (CTAs) per chain
   int ksplit, n_eh, dx_bn;
-  bool dx_pair;             // CTA-pair dx kernel (row count a multiple of 512)
+  bool dx_pair;             // CTA-pair dx kernel (row blocks a multiple of 4; the last one may be partial)
   size_t g_bytes, g_buf_bytes, dxp_bytes;
 };
 

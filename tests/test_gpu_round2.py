@@ -118,6 +118,8 @@ def test_range_guard_every_step(pkg):
     assert abs(float(loss) - float(ref.loss)) <= 3e-2 * float(ref.loss)
     assert rel(xg.cpu(), ref.x_grad[0]) < 3e-2 and rel(head.sub_weight.grad.cpu(), ref.dw[0]) < 3e-2
     head._ops.bwd_mode = "prob"                                        # shared per-device provider: leave it as found
+    for slot in range(4):                                              # and the per-device flag pairs too: a pair raised
+        head._ops.read_range_slot(slot)                                # here and never read would switch a later head
 
 
 def test_fedavg_signed_zero_unaligned_and_many_clients(pkg):
