@@ -12,6 +12,7 @@
 // or below the diagonal are skipped.  The bound is the fp32-multiply / convert / fp64-add chain per (pair, k), not HBM:
 // a 64 x 64 tile reads 2 * 64 * emb * 4 bytes for 4096 * emb such chains.
 #include "common.cuh"
+#include "../../fedfr_b200/csrc/dot_chain.cuh"
 
 namespace pfc {
 
@@ -125,9 +126,7 @@ roc_hist_kernel(const float* __restrict__ feature, const int32_t* __restrict__ l
 constexpr int kRocQueue = 1024;
 
 __device__ __forceinline__ double roc_exact_x(const float* __restrict__ a, const float* __restrict__ b, int emb) {
-  double tmp = 0.0;
-  for (int k = 0; k < emb; ++k) tmp = __dadd_rn(tmp, (double)__fmul_rn(a[k], b[k]));
-  return __dmul_rn(__dadd_rn(tmp, 1.0), 1000.0);
+  return __dmul_rn(__dadd_rn(dot_chain(0.0, a, b, emb), 1.0), 1000.0);
 }
 
 // Exact chain for every queued pair, one pair per thread.  Called by the whole CTA (barriers inside); q_n may exceed the

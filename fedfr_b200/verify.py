@@ -1,0 +1,157 @@
+"""1:1 template verification on the sm_100a kernels -- the IJB-B / IJB-C protocol of FedFR's ``ijbc_all.py`` /
+``ijbc_conti.py``, on arrays: image features with template and media ids, a template pair list, genuine flags.
+
+    template_feats, template_ids = template_features(feats, templates, medias, weights)
+    scores = pair_scores(template_feats, template_ids, p1, p2)
+    for far_target, tar, far, threshold in tar_at_far(scores, issame): ...
+
+The arithmetic is this repository's definition, pinned step by step (``include/fedfr_b200.h``, ``csrc/verify.cu``) so that
+a plain C restatement reproduces every feature and score bit for bit; it follows the usual insightface recipe (media
+mean, template sum, L2 normalise, cosine).  Inputs are CUDA tensors or numpy arrays; nothing runs on the CPU except
+index plumbing on the device (sorting ids into a CSR, id -> row lookup) and the final division of two counts.
+"""
+import numpy as np
+import torch
+
+from . import _native as N
+
+DEFAULT_FARS = (1e-6, 1e-5, 1e-4, 1e-3, 1e-2, 1e-1)
+_MAX_FARS_PER_CALL = 8
+
+
+def _device(t):
+    if isinstance(t, torch.Tensor) and t.is_cuda:
+        return t.device
+    return torch.device("cuda", torch.cuda.current_device())
+
+
+def _on(t, dtype, device):
+    if isinstance(t, np.ndarray):
+        t = torch.from_numpy(np.ascontiguousarray(t))
+    return torch.as_tensor(t).to(device=device, dtype=dtype).contiguous()
+
+
+def _stream(device):
+    return torch.cuda.current_stream(device).cuda_stream
+
+
+def pool_index(templates, medias):
+    """CSR of the images in ascending (template, media, row) order, from int64 id tensors on any device:
+    -> (template_ids [T], order [n], media_start [n_media + 1], tmpl_start [T + 1])."""
+    template_ids, t_inv = torch.unique(templates, return_inverse=True)
+    media_ids, m_inv = torch.unique(medias, return_inverse=True)
+    key = t_inv * media_ids.numel() + m_inv
+    key_sorted, order = torch.sort(key, stable=True)
+    _, counts = torch.unique_consecutive(key_sorted, return_counts=True)
+    media_start = torch.cat([counts.new_zeros(1), counts.cumsum(0)])
+    media_tmpl = key_sorted[media_start[:-1]] // media_ids.numel()
+    tmpl_start = torch.searchsorted(media_tmpl, torch.arange(template_ids.numel() + 1, device=key.device))
+    return template_ids, order, media_start, tmpl_start
+
+
+def template_features(feats, templates, medias, weights=None):
+    """Pool image features into L2-normalised template features.
+
+    feats fp32 [n, E]; templates, medias int64 [n] (arbitrary ids; a media is a (template, media) pair, so one media id
+    may occur in several templates); weights fp32 [n] or None (a per-image scale such as a detector score).  Each media
+    is the mean of its images, each template the sum of its medias (ascending media id), then normalised.
+    -> (template_feats fp32 [T, E], template_ids int64 [T], sorted unique), on the GPU."""
+    device = _device(feats)
+    f = _on(feats, torch.float32, device)
+    t = _on(templates, torch.int64, device).reshape(-1)
+    m = _on(medias, torch.int64, device).reshape(-1)
+    w = None if weights is None else _on(weights, torch.float32, device).reshape(-1)
+    if f.dim() != 2 or f.shape[0] == 0 or f.shape[1] == 0:
+        raise ValueError("feats must be a non-empty [n, E] array")
+    n, emb = f.shape
+    if t.numel() != n or m.numel() != n or (w is not None and w.numel() != n):
+        raise ValueError("templates, medias and weights need one entry per image row")
+    template_ids, order, media_start, tmpl_start = pool_index(t, m)
+    out = torch.empty(template_ids.numel(), emb, dtype=torch.float32, device=device)
+    with torch.cuda.device(device):
+        N.check(N.lib.pfc_template_pool(N.ptr(f), N.ptr(w), N.ptr(order), N.ptr(media_start), N.ptr(tmpl_start),
+                                        template_ids.numel(), emb, N.ptr(out), _stream(device)), "pfc_template_pool")
+    return out, template_ids
+
+
+def pair_rows(template_ids, p1, p2):
+    """Template ids -> rows of ``template_ids`` (sorted unique), by binary search on the ids' device.  ValueError for an
+    id that is not there."""
+    if template_ids.numel() == 0 or bool((template_ids[1:] <= template_ids[:-1]).any()):
+        raise ValueError("template_ids must be non-empty, sorted and unique (as template_features returns them)")
+    rows = []
+    for p in (p1, p2):
+        r = torch.searchsorted(template_ids, p).clamp_(max=template_ids.numel() - 1)
+        missing = template_ids[r] != p
+        if bool(missing.any()):
+            raise ValueError("unknown template id %d in the pair list" % int(p[missing.nonzero()[0, 0]]))
+        rows.append(r)
+    return rows
+
+
+def pair_scores(template_feats, template_ids, p1, p2):
+    """Cosine of each template pair: ``sum_k (double)fl32(a_k * b_k)`` over ascending k, rounded to fp32 (the chain of
+    the ROC histogram).  template_feats fp32 [T, E] and template_ids int64 [T] as template_features returns them;
+    p1, p2 int64 [P] template ids.  Pair lists grouped by p1 (as IJB-C's is) read each p1 row once per 128 pairs.
+    -> scores fp32 [P] on the GPU."""
+    device = _device(template_feats)
+    tf = _on(template_feats, torch.float32, device)
+    ids = _on(template_ids, torch.int64, device).reshape(-1)
+    a = _on(p1, torch.int64, device).reshape(-1)
+    b = _on(p2, torch.int64, device).reshape(-1)
+    if tf.dim() != 2 or tf.shape[0] != ids.numel():
+        raise ValueError("template_feats [T, E] needs one id per row")
+    if a.numel() != b.numel():
+        raise ValueError("p1 and p2 must have the same length")
+    out = torch.empty(a.numel(), dtype=torch.float32, device=device)
+    if a.numel() == 0:
+        return out
+    r1, r2 = pair_rows(ids, a, b)
+    with torch.cuda.device(device):
+        N.check(N.lib.pfc_pair_scores(N.ptr(tf), tf.shape[0], tf.shape[1], N.ptr(r1), N.ptr(r2), a.numel(), N.ptr(out),
+                                      _stream(device)), "pfc_pair_scores")
+    return out
+
+
+def tar_from_counts(counts, thresholds, fars):
+    """(counts [3 + 2 n_far] of pfc_tar_at_far, thresholds [n_far]) -> [(far_target, tar, far, threshold)]."""
+    counts = [int(c) for c in counts]
+    n_gen, n_imp, n_nan = counts[:3]
+    if n_nan:
+        raise ValueError("%d scores are NaN" % n_nan)
+    if n_gen == 0 or n_imp == 0:
+        raise ValueError("tar_at_far needs genuine and impostor pairs (got %d and %d)" % (n_gen, n_imp))
+    return [(float(f), counts[3 + 2 * q] / n_gen, counts[4 + 2 * q] / n_imp, float(thresholds[q])) for q, f in enumerate(fars)]
+
+
+def tar_at_far(scores, issame, fars=DEFAULT_FARS):
+    """Exact TAR at each target FAR from the full score distribution (no sort, no binning).
+
+    With n_imp impostor pairs and k = floor(f * n_imp), the threshold is the (k+1)-th largest impostor score (-inf when
+    k >= n_imp) and a pair is accepted iff its score is above it, so ties at the threshold are rejected and the achieved
+    far = accepted impostors / n_imp is at most f: the best operating point with FAR <= f.  -0.0 and +0.0 are one
+    value.  The sklearn-based IJB scripts instead read the nearest point of a thinned ROC curve; that lookup is not
+    reproduced.  scores fp32 [P], issame bool [P]; fars in (0, 1].  A NaN score, or no genuine or no impostor pair,
+    raises ValueError.  -> [(far_target, tar, far, threshold)]."""
+    device = _device(scores)
+    s = _on(scores, torch.float32, device).reshape(-1)
+    y = (_on(issame, torch.int64, device).reshape(-1) != 0).to(torch.uint8)
+    fars = [float(f) for f in fars]
+    if s.numel() != y.numel():
+        raise ValueError("one issame flag per score")
+    if s.numel() == 0:
+        raise ValueError("tar_at_far needs genuine and impostor pairs (got no scores)")
+    if not fars or not all(0.0 < f <= 1.0 for f in fars):
+        raise ValueError("FARs must lie in (0, 1]")
+    ws = torch.empty(int(N.lib.pfc_tar_at_far_workspace_bytes(s.numel())), dtype=torch.uint8, device=device)
+    result = []
+    for c0 in range(0, len(fars), _MAX_FARS_PER_CALL):
+        chunk = fars[c0:c0 + _MAX_FARS_PER_CALL]
+        f_host = np.asarray(chunk, dtype=np.float64)
+        counts = torch.empty(3 + 2 * len(chunk), dtype=torch.int64, device=device)
+        thr = torch.empty(len(chunk), dtype=torch.float32, device=device)
+        with torch.cuda.device(device):
+            N.check(N.lib.pfc_tar_at_far(N.ptr(s), N.ptr(y), s.numel(), f_host.ctypes.data, len(chunk), N.ptr(counts),
+                                         N.ptr(thr), N.ptr(ws), ws.numel(), _stream(device)), "pfc_tar_at_far")
+        result += tar_from_counts(counts.cpu().tolist(), thr.cpu().tolist(), chunk)
+    return result

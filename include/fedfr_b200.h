@@ -287,6 +287,36 @@ int pfc_similar_columns(const float* a, int64_t n_a, const float* b, int64_t n_b
 int pfc_roc_histogram(const float* feature, const int32_t* label, int64_t n, const float* subfeature,
                       const int32_t* sublabel, int64_t n_sub, int64_t sub_offset, int emb, int64_t* hist, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * 1:1 template verification (IJB-B / IJB-C protocol)         ijbc_all.py / ijbc_conti.py
+ * ------------------------------------------------------------------------------------------------
+ * Template pooling.  feats fp32 [n, emb] (emb <= 4096), weights fp32 [n] or NULL (a per-image scale).  The images are
+ * given in ascending (template, media, row) order as a CSR: order int64 [n] lists image rows, media j holds
+ * order[media_start[j] .. media_start[j+1]), template t holds medias tmpl_start[t] .. tmpl_start[t+1]
+ * (media_start [n_media + 1], tmpl_start [n_templates + 1], both ascending, every media non-empty; fedfr_b200.verify
+ * builds them).  Writes template_feats fp32 [n_templates, emb]:
+ *     x = feats_i (* weights_i, fp32);  media = fp32 sum of its images in order, / (float)count when count > 1;
+ *     t = fp32 sum of the medias in order;  out_k = (float)((double)t_k / max(sqrt(sum_k (double)t_k^2), 1e-12)).
+ * Deterministic (no atomics). */
+int pfc_template_pool(const float* feats, const float* weights, const int64_t* order, const int64_t* media_start,
+                      const int64_t* tmpl_start, int64_t n_templates, int emb, float* template_feats, void* stream);
+
+/* scores[p] = (float)(sum_k (double)fl32(a_k * b_k)), k ascending, a = template_feats[row1[p]], b = template_feats[row2[p]]
+ * (the pfc_roc_histogram chain).  A pair with a row outside [0, n_templates) scores NaN.  Pairs grouped by row1 read
+ * that row once per 128 pairs. */
+int pfc_pair_scores(const float* template_feats, int64_t n_templates, int emb, const int64_t* row1, const int64_t* row2,
+                    int64_t n_pairs, float* scores, void* stream);
+
+/* Exact TAR@FAR without sorting.  scores fp32 [n] (n < 2^31), issame uint8 [n] (nonzero = genuine); fars_host: n_far
+ * (1..8) host doubles in (0, 1].  With n_imp impostors and k = floor(f * n_imp) (fp64), the threshold is the (k+1)-th
+ * largest impostor score (-inf when k >= n_imp) and a pair is accepted iff score > threshold (-0.0 == +0.0).  Writes
+ * counts int64 [3 + 2 n_far] = {n_gen, n_imp, n_nan, then accepted genuine, accepted impostor per FAR} and thresholds
+ * fp32 [n_far]; NaN scores are counted in n_nan and in no class.  workspace: pfc_tar_at_far_workspace_bytes(n) bytes,
+ * 8-byte aligned. */
+size_t pfc_tar_at_far_workspace_bytes(int64_t n);
+int pfc_tar_at_far(const float* scores, const unsigned char* issame, int64_t n, const double* fars_host, int n_far,
+                   int64_t* counts, float* thresholds, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
