@@ -192,7 +192,7 @@ int pfc_set_debug_buffer(void* dev_ptr) {
  * row sum is 0 / non-finite in pfc_bwd_prob.  Sticky; applies to the calling thread's current device. */
 int pfc_set_range_flag(int* flag, float limit_nats) { return tc_set_range_flag(flag, limit_nats); }
 
-int pfc_set_dw4(int on) {   /* E = 512 dw kernel: -1 auto (default), 0 e-split pair kernel, 1 / 2 the 4-CTA-cluster kernel (multicast / independent pairs) */
+int pfc_set_dw4(int on) {   /* E = 512 dw kernel: -1 auto (default), 0 e-split pair kernel, > 0 the 4-CTA-cluster kernel */
   tc_set_dw4(on);
   return 0;
 }

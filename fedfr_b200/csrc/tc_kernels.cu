@@ -109,7 +109,6 @@ struct LogitsParams {
   // MODE_PROB (forward that keeps the unnormalised probabilities): P_ij = exp2(s2 cos_ij - row_bound_i) -> bf16 scratch
   const float* row_bound;    // [n_rows] log2 units: an upper bound of every logit of the row minus a fixed headroom
   float* target_cos;         // [n_rows] plain cosine at the target column (the backward's fp32 fix-up needs it)
-  int exp;                   // timing experiments only (FEDFR_FWD_EXP, wrong results): 1 no ex2, 2 no P store
 };
 
 __device__ __forceinline__ float fast_exp2(float x) {
@@ -693,7 +692,7 @@ __global__ void __launch_bounds__(kLogitsThreads + (NORM ? norm_warps(MODE) * 32
 #pragma unroll
           for (int q = 0; q < 16; ++q) {
             const float2 zz = __ffma2_rn(make_float2(__uint_as_float(v[2 * q]), __uint_as_float(v[2 * q + 1])), s2v, m2v);
-            g[q] = (p.exp & 1) ? zz : make_float2(fast_exp2(zz.x), fast_exp2(zz.y));
+            g[q] = make_float2(fast_exp2(zz.x), fast_exp2(zz.y));
           }
           if (tile_has_oob) {
 #pragma unroll
@@ -728,7 +727,7 @@ __global__ void __launch_bounds__(kLogitsThreads + (NORM ? norm_warps(MODE) * 32
             fence_proxy_async_smem();
             __syncwarp();
             const int cbg = p.class_base + cb;               // the scratch spans the whole shard
-            if (lane == 0 && cbg < p.ldg && rb < p.n_rb && !(p.exp & 2)) {
+            if (lane == 0 && cbg < p.ldg && rb < p.n_rb) {
               tma_store_2d(&tmap_g, gbuf, 0, ((cbg >> 6) * p.n_rb + rb) * BM + quad * 32);
               tma_store_commit();
             }
@@ -1156,7 +1155,6 @@ struct DwParams {
   int accumulate;
   int prefetch;                   // 1: TMA L2 prefetch of the next tile's G / w_hat boxes
   long long* dbg;                 // optional cycle counters of CTA 0 (developer instrumentation), else nullptr
-  int exp;                        // timing experiments only (FEDFR_DW_EXP, wrong results): 1 no pass 1, 2 no exchange, 4 no pass 2 / stores, 8 no w_hat loads
 };
 
 __device__ __forceinline__ void st_cluster_f32(uint32_t cluster_addr, float v) {
@@ -1166,14 +1164,8 @@ __device__ __forceinline__ void st_cluster_f32(uint32_t cluster_addr, float v) {
 constexpr int kDwEpiWarps = 8;                 // two warps per TMEM lane quadrant, each takes half of the slice's columns
 constexpr int kDwThreads = (kDwEpiWarps + 2) * 32;
 
-// P2 (E = 512 only, cluster of 4): the same kernel on cta_group::2 pairs.  Pair h = cluster ranks (2h, 2h+1) computes e-slice
-// h of TWO class tiles with one M = 256 MMA (CTA of parity c: tile 2g + c, and the N-half c of x_scaled), so a CTA fills 32 KB
-// per k-block instead of 48 and reads 8 KB of operands per MMA instead of 12 (section 5a of DESIGN.md); the partial dots
-// are exchanged with the CTA that owns the same class tile in the other pair (rank ^ 2).  Epilogue unchanged.
-// EW = epilogue warps: 8 (two column halves per lane quadrant) or 16 (four column groups: half the serial chain per warp --
-// tcgen05.ld, fma, st.shared, proxy fence, TMA store per 32-column group -- which is what bounds the kernel at small K).
-template <int EMB, int STAGES, int CS, bool P2 = false, int EW = kDwEpiWarps>
-__global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_constant__ CUtensorMap tmap_x,
+template <int EMB, int STAGES, int CS>
+__global__ void __launch_bounds__(kDwThreads, 1) dw_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_constant__ CUtensorMap tmap_x,
                                                            const __grid_constant__ CUtensorMap tmap_wh, const __grid_constant__ CUtensorMap tmap_dw,
                                                            const DwParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -1181,60 +1173,52 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
   constexpr int EN = EMB < 256 ? EMB : 256;              // accumulator width = N of one MMA
   constexpr int NH = EMB / EN;                           // e-slices per class tile
   constexpr bool ES = NH == 2;                           // e-split cluster: both CTAs work on the same class tile
-  static_assert(!ES || (!P2 && CS == 2) || (P2 && CS == 4), "the e-split arrangement is a cluster of two CTAs (four with cta_group::2 pairs)");
-  static_assert(!P2 || ES, "pairs of pairs only for E = 512");
+  static_assert(!ES || CS == 2, "the e-split arrangement is a cluster of two CTAs");
   constexpr int NBOX = EN / 64;                          // 64-wide boxes per e-slice
-  constexpr int NCG = EW / 4;                            // column groups (epilogue warps per lane quadrant)
+  constexpr int NCG = kDwEpiWarps / 4;                   // column groups (epilogue warps per lane quadrant)
   constexpr int CW = EN / NCG;                           // columns per epilogue warp
   constexpr int NG = CW / 32;                            // 32-column groups per epilogue warp (1, 2 or 4)
   constexpr int kContrib = (ES ? 2 : 1) * NCG;           // partial dots per class row: (cluster rank x) column group
-  static_assert(CW >= 32 && kContrib <= 8, "epilogue warp count");
   constexpr int kABytes = 2 * kBoxBytes;                 // 128 classes x 64 rows
-  constexpr int kBBytes = P2 ? 2 * kBoxBytes : NBOX * kBoxBytes;      // EN x 64 rows (P2: this CTA's 128-e half of it)
+  constexpr int kBBytes = NBOX * kBoxBytes;              // EN x 64 rows
   constexpr int kStageBytes = kABytes + kBBytes;
   constexpr int kWBox = 32 * 128;                        // w_hat box: 32 classes x 64 e bf16 = 4 KB = one fp32 staging box [32 x 32]
   constexpr int kWWarp = (NG + 1) / 2 * kWBox;           // per-warp w_hat columns (a warp with 32 columns still loads a 64-e box)
-  constexpr bool kDeep = P2 && NG == 4;                  // a third staging box per warp: three output stores in flight instead of two
-  constexpr int kSBox = NG == 1 ? 2 : (kDeep ? 1 : 0);   // extra staging boxes (warps that own a single w_hat box; the deep pipeline)
+  constexpr int kSBox = NG == 1 ? 2 : 0;                 // extra staging boxes of the warps that own a single w_hat box
   uint8_t* smem_w = smem + STAGES * kStageBytes;         // [8 warps] w_hat boxes, reused as output staging
-  uint8_t* smem_s = smem_w + EW * kWWarp;                // [EW warps][kSBox] staging
-  float* tpart = reinterpret_cast<float*>(smem_s + EW * kSBox * kWBox);   // [2][kContrib][128] partial dots
+  uint8_t* smem_s = smem_w + kDwEpiWarps * kWWarp;       // [8 warps][kSBox] staging
+  float* tpart = reinterpret_cast<float*>(smem_s + kDwEpiWarps * kSBox * kWBox);   // [2][kContrib][128] partial dots
   uint64_t* bars = reinterpret_cast<uint64_t*>(tpart + 2 * 8 * 128);
   uint64_t* full = bars;
   uint64_t* empty = bars + STAGES;
   uint64_t* tmem_full = bars + 2 * STAGES;               // [2]
   uint64_t* tmem_empty = bars + 2 * STAGES + 2;          // [2]
-  uint64_t* wfull = bars + 2 * STAGES + 4;               // [EW warps]
-  uint64_t* tbar = bars + 2 * STAGES + 4 + EW;           // [2][4 quadrants] all partial dots of the quadrant's rows have landed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 12 + EW);
+  uint64_t* wfull = bars + 2 * STAGES + 4;               // [8 warps]
+  uint64_t* tbar = bars + 2 * STAGES + 4 + kDwEpiWarps;  // [2][4 quadrants] all partial dots of the quadrant's rows have landed
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 12 + kDwEpiWarps);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_kb = (p.n_rows + BK - 1) / BK;
   const uint32_t crank = CS > 1 ? cluster_ctarank() : 0;
   const int n_clusters = gridDim.x / CS, cid = blockIdx.x / CS;
   constexpr uint16_t kMask = (uint16_t)((1u << CS) - 1);
-  constexpr int kProducerWarp = EW, kMmaWarp = EW + 1;
+  constexpr int kProducerWarp = kDwEpiWarps, kMmaWarp = kDwEpiWarps + 1;
   // ES:   item i -> class tile i * n_clusters + cid (both CTAs), e-slice = cluster rank.
   // else: item i -> class tile (i * n_clusters + cid) * CS + crank, the only e-slice.  Every CTA of a cluster runs the
   //       same number of items (tiles past n_ct are phantoms: TMA zero-fills their loads and clips their stores).
-  // P2:   item i -> class tiles 2 (i * n_clusters + cid) + parity; e-slice = pair index.
-  const int cpar = P2 ? (int)(crank & 1) : 0;
-  auto tile_of = [&](int i) { return P2 ? 2 * (i * n_clusters + cid) + cpar : (ES ? i * n_clusters + cid : (i * n_clusters + cid) * CS + (int)crank); };
-  auto more = [&](int i) { return P2 ? 2 * (i * n_clusters + cid) < p.n_ct : (ES ? i * n_clusters + cid < p.n_ct : (i * n_clusters + cid) * CS < p.n_ct); };
-  const int hs = P2 ? (int)(crank >> 1) : (ES ? (int)crank : 0);
-  const bool mma_leader = !P2 || cpar == 0;
-  const uint32_t leader_rank = crank & ~1u;
-  const uint16_t pair_mask = (uint16_t)(3u << (2 * hs));
+  auto tile_of = [&](int i) { return ES ? i * n_clusters + cid : (i * n_clusters + cid) * CS + (int)crank; };
+  auto more = [&](int i) { return ES ? i * n_clusters + cid < p.n_ct : (i * n_clusters + cid) * CS < p.n_ct; };
+  const int hs = ES ? (int)crank : 0;
 
   if (threadIdx.x == 0) {
-    for (int i = 0; i < STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], P2 ? 1 : CS); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], P2 ? 2 * EW : EW); }
-    for (int i = 0; i < EW; ++i) mbar_init(&wfull[i], 1);
+    for (int i = 0; i < STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], CS); }
+    for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], kDwEpiWarps); }
+    for (int i = 0; i < kDwEpiWarps; ++i) mbar_init(&wfull[i], 1);
     for (int i = 0; i < 8; ++i) mbar_init(&tbar[i], kContrib);
     fence_barrier_init();
   }
   if (warp == kProducerWarp && lane == 0) { prefetch_tmap(&tmap_g); prefetch_tmap(&tmap_x); prefetch_tmap(&tmap_wh); prefetch_tmap(&tmap_dw); }
-  if (warp == kMmaWarp) { if (P2) tmem_alloc_2cta<2 * EN>(tmem_slot); else tmem_alloc<2 * EN>(tmem_slot); }
+  if (warp == kMmaWarp) tmem_alloc<2 * EN>(tmem_slot);
   tc_fence_before();
   if (CS > 1) cluster_sync_all(); else __syncthreads();
   tc_fence_after();
@@ -1250,17 +1234,6 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
           mbar_wait_cluster(&empty[ps.stage], ps.phase ^ 1);
           uint8_t* sa = smem + ps.stage * kStageBytes;
           uint8_t* sb = sa + kABytes;
-          if (P2) {                               // both CTAs of the pair credit the leader's barrier (dx2's producer)
-            const uint32_t full_leader = mapa_u32(smem_u32(&full[ps.stage]), leader_rank);
-            if (mma_leader) mbar_arrive_expect_tx(&full[ps.stage], 2 * kStageBytes);
-#pragma unroll
-            for (int hb = 0; hb < 2; ++hb)
-              tma_load_2d_2cta(sa + hb * kBoxBytes, &tmap_g, full_leader, 0, ((2 * ct + hb) * p.n_rb + (kb >> 1)) * BM + (kb & 1) * 64);
-#pragma unroll
-            for (int nb = 0; nb < 2; ++nb) tma_load_2d_2cta(sb + nb * kBoxBytes, &tmap_x, full_leader, hs * EN + cpar * 128 + nb * 64, kb * BK);
-            ps.advance(STAGES);
-            continue;
-          }
           mbar_arrive_expect_tx(&full[ps.stage], kStageBytes);
           // G scratch blocks (2 ct, kb / 2) and (2 ct + 1, kb / 2): 64 rows x 64 classes each, contiguous 8 KB
           if (ES) {                               // this CTA fetches class half `crank` for both CTAs of the cluster
@@ -1287,8 +1260,8 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
       }
     }
   } else if (warp == kMmaWarp) {
-    if (lane == 0 && mma_leader) {
-      constexpr uint32_t idesc = make_idesc_bf16(P2 ? 2 * BM : BM, EN, true, true);
+    if (lane == 0) {
+      constexpr uint32_t idesc = make_idesc_bf16(BM, EN, true, true);
       PipeState ps;
       long long t_we = 0, t_wf = 0, t_all = clock64();
       for (int it = 0; more(it); ++it) {
@@ -1309,15 +1282,13 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
           for (int kk = 0; kk < BK / 16; ++kk) {
             const uint64_t da = make_desc_sw128(a_addr + kk * 2048, kBoxBytes, 1024);
             const uint64_t db = make_desc_sw128(b_addr + kk * 2048, kBoxBytes, 1024);
-            if (P2) umma_bf16_ss_2cta(d_tmem, da, db, idesc, (kb | kk) != 0);
-            else umma_bf16_ss(d_tmem, da, db, idesc, (kb | kk) != 0);
+            umma_bf16_ss(d_tmem, da, db, idesc, (kb | kk) != 0);
           }
-          if (P2) umma_commit_2cta(&empty[ps.stage], pair_mask);
-          else if (CS == 1) umma_commit(&empty[ps.stage]);
+          if (CS == 1) umma_commit(&empty[ps.stage]);
           else umma_commit_mc(&empty[ps.stage], kMask);
           ps.advance(STAGES);
         }
-        if (P2) umma_commit_2cta(&tmem_full[acc], pair_mask); else umma_commit(&tmem_full[acc]);
+        umma_commit(&tmem_full[acc]);
       }
       if (p.dbg && blockIdx.x == 0) { p.dbg[0] = t_we; p.dbg[1] = t_wf; p.dbg[2] = clock64() - t_all; }
     }
@@ -1330,9 +1301,8 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
     uint8_t* wbuf = smem_w + warp * kWWarp;
     uint8_t* sbuf = smem_s + warp * kSBox * kWBox;
     uint64_t* wbar = &wfull[warp];
-    const uint32_t peer = P2 ? crank ^ 2u : crank ^ 1u;    // the CTA holding the other e-slice of the same class tile
+    const uint32_t peer = crank ^ 1u;                     // the CTA holding the other e-slice of the same class tile
     const int contrib = (ES ? hs * NCG : 0) + chalf;
-    const uint32_t tmem_leader_empty0 = mapa_u32(smem_u32(&tmem_empty[0]), leader_rank);
     const int e_warp = hs * EN + chalf * CW;              // first e column of this warp
     long long t_wfull = 0, t_ww = 0, t_ep = 0, t_p1 = 0, t_ex = 0, t_p2 = 0;
     auto issue_w = [&](int i) {                           // this warp's w_hat rows of item i (lane 0 only)
@@ -1348,8 +1318,7 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
     };
     constexpr int kSub = NG == 1 ? 4 : 0;                 // 32-column warps read the upper / lower half of their 64-e box
     const int sub0 = NG == 1 ? ((e_warp >> 5) & 1) * kSub : 0;
-    const int ex = p.exp;
-    if (lane == 0 && more(0) && !(ex & 8)) issue_w(0);
+    if (lane == 0 && more(0)) issue_w(0);
     for (int it = 0; more(it); ++it) {
       const int ct = tile_of(it);
       const int acc = it & 1;
@@ -1361,7 +1330,7 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
       mbar_wait(&tmem_full[acc], (uint32_t)((it >> 1) & 1));
       t_wfull += clock64() - c0;
       c0 = clock64();
-      if (!(ex & 8)) mbar_wait(wbar, (uint32_t)(it & 1));
+      mbar_wait(wbar, (uint32_t)(it & 1));
       t_ww += clock64() - c0;
       c0 = clock64();
       tc_fence_after();
@@ -1381,7 +1350,6 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
                                 make_float2(__uint_as_float(v[q * 8 + 2 * k]), __uint_as_float(v[q * 8 + 2 * k + 1])), dot2);
           }
         };
-        if (!(ex & 1)) {
         tmem_ld_x32(t_base, va);
 #pragma unroll
         for (int g = 0; g < NG; g += 2) {
@@ -1394,28 +1362,24 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
             dot_group(vb, g + 1);
           }
         }
-        }
       }
       t_p1 += clock64() - c0;
       // ---- exchange: every contributor (column half x cluster rank) publishes its partial to each CTA that needs it
-      float t = 0.f;
-      if (!(ex & 2)) {
-        const int buf = it & 1;
-        float* slot = tpart + (buf * 8 + contrib) * 128 + quad * 32 + lane;
-        *slot = dot2.x + dot2.y;
-        if (ES) st_cluster_f32(mapa_u32(smem_u32(slot), peer), dot2.x + dot2.y);
-        __syncwarp();                                     // one release per warp covers the 32 lanes' stores (not 32 cluster fences)
-        if (lane == 0) {
-          mbar_arrive(&tbar[buf * 4 + quad]);
-          if (ES) mbar_arrive_remote(&tbar[buf * 4 + quad], peer);
-        }
-        if (ES) mbar_wait_cluster(&tbar[buf * 4 + quad], (uint32_t)((it >> 1) & 1));
-        else mbar_wait(&tbar[buf * 4 + quad], (uint32_t)((it >> 1) & 1));
-        const float* all = tpart + buf * 8 * 128 + quad * 32 + lane;
-        t = all[0];                                       // fixed order: every warp (and both CTAs) get the same bits
-#pragma unroll
-        for (int c = 1; c < kContrib; ++c) t += all[c * 128];
+      const int buf = it & 1;
+      float* slot = tpart + (buf * 8 + contrib) * 128 + quad * 32 + lane;
+      *slot = dot2.x + dot2.y;
+      if (ES) st_cluster_f32(mapa_u32(smem_u32(slot), peer), dot2.x + dot2.y);
+      __syncwarp();                                       // one release per warp covers the 32 lanes' stores (not 32 cluster fences)
+      if (lane == 0) {
+        mbar_arrive(&tbar[buf * 4 + quad]);
+        if (ES) mbar_arrive_remote(&tbar[buf * 4 + quad], peer);
       }
+      if (ES) mbar_wait_cluster(&tbar[buf * 4 + quad], (uint32_t)((it >> 1) & 1));
+      else mbar_wait(&tbar[buf * 4 + quad], (uint32_t)((it >> 1) & 1));
+      const float* all = tpart + buf * 8 * 128 + quad * 32 + lane;
+      float t = all[0];                                   // fixed order: every warp (and both CTAs) get the same bits
+#pragma unroll
+      for (int c = 1; c < kContrib; ++c) t += all[c * 128];
       t_ex += clock64() - c0;
       const float c1 = ok ? -t * inv_n : 0.f;
       const float2 c1v = make_float2(c1, c1), inv2 = make_float2(inv_n, inv_n);
@@ -1429,15 +1393,11 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
       {
         uint32_t va[32];
         auto out_group = [&](const uint32_t (&v)[32], int g) {
-          // kDeep: groups 0..3 -> boxes (extra, w_hat box 0, w_hat box 1, extra): the extra box was last used three groups ago,
-          // the w_hat boxes were reloaded (and read into registers) since their last store -- almost nothing to wait for
-          uint8_t* orow = NG == 1 ? sbuf + (it & 1) * kWBox : (kDeep ? ((g == 0 || g == 3) ? sbuf : wbuf + (g - 1) * kWBox) : wbuf + (g & (kNW - 1)) * kWBox);
+          uint8_t* orow = NG == 1 ? sbuf + (it & 1) * kWBox : wbuf + (g & (kNW - 1)) * kWBox;
           // the store issued two groups ago (same box) must have been read; stores are committed one group each
           if (lane == 0) {
             if (NG == 1) tma_store_wait_read<1>();
-            else if (!kDeep) tma_store_wait_read<kNW - 1>();
-            else if (g == 0) tma_store_wait_read<0>();
-            else if (g == 3) tma_store_wait_read<2>();
+            else tma_store_wait_read<kNW - 1>();
           }
           __syncwarp();
 #pragma unroll
@@ -1460,24 +1420,20 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
             tma_store_commit();
           }
         };
-        if (!(ex & 4)) {
 #pragma unroll
         for (int g = 0; g < NG; ++g) {                    // (one group in flight: the 16 w_hat registers leave no room for two)
           tmem_ld_x32(t_base + g * 32, va);
           tmem_ld_wait();
           out_group(va, g);
         }
-        }
       }
       t_p2 += clock64() - c0;
       tc_fence_before();
       __syncwarp();
       if (lane == 0) {
-        if (mma_leader) mbar_arrive(&tmem_empty[acc]);
-        else mbar_arrive_cluster_addr_relaxed(tmem_leader_empty0 + acc * 8);
-        if (kDeep) tma_store_wait_read<1>();              // the w_hat boxes carried groups 1 and 2; group 3 (extra box) may still be read
-        else if (NG > 1) tma_store_wait_read<0>();        // the staging boxes are this warp's w_hat boxes: all reads done before the reload
-        if (more(it + 1) && !(ex & 8)) issue_w(it + 1);
+        mbar_arrive(&tmem_empty[acc]);
+        if (NG > 1) tma_store_wait_read<0>();             // the staging boxes are this warp's w_hat boxes: all reads done before the reload
+        if (more(it + 1)) issue_w(it + 1);
       }
       __syncwarp();
       t_ep += clock64() - c0;
@@ -1487,7 +1443,7 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
   }
   tc_fence_before();
   if (CS > 1) cluster_sync_all(); else __syncthreads();     // peers may still multicast into / arrive on this CTA
-  if (warp == kMmaWarp) { if (P2) tmem_dealloc_2cta<2 * EN>(tmem_base); else tmem_dealloc<2 * EN>(tmem_base); }
+  if (warp == kMmaWarp) tmem_dealloc<2 * EN>(tmem_base);
 }
 
 // ================================================================================================
@@ -1500,9 +1456,8 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
 // L1 data pipe, which TMA fills, tcgen05.mma operand reads, ld/st.shared AND every global load/store wavefront share.  In
 // 128-byte slots per 4096-cycle item the e-split pair kernel above needs 3072 (fill) + 3072 (cta_group::1 operand reads)
 // + 3584 (w_hat boxes, fp32 staging, TMA store) = 9728 -> 42 % of the tensor rate, which is what it measures.  Here:
-//   * cta_group::2 halves the operand reads per CTA (2048 slots) and the B fill;
-//   * the P tile of a class tile is needed by the same-parity CTA of BOTH pairs: each loads one 64-class box and
-//     multicasts it to the other (1024 slots of fill, 8 KB from L2 per CTA per k-block);
+//   * cta_group::2 halves the operand reads per CTA (2048 slots) and the B fill (1024 slots, 16 KB from L2 per CTA per
+//     k-block);
 //   * x_scaled^T, the M-side operand, is the SAME for every item: with Bt <= 512 its [512 rows x 128 e] slice (128 KB)
 //     stays resident in shared memory (STAT, no fill at all); larger batches stream it (16 KB per k-block);
 //   * lane = e means a warp's 32 lanes hold 32 CONSECUTIVE e of one class per register: dw leaves in full 128-byte
@@ -1511,9 +1466,10 @@ __global__ void __launch_bounds__((EW + 2) * 32, 1) dw_kernel(const __grid_const
 //   * the radial term t_j = w_hat_j . dW_hat_j is a sum over e = over lanes: a shuffle transpose-reduction per 32 x 32
 //     block (warp_colsum32), then over the 4 lane quadrants (shared memory) and the 4 CTAs (DSMEM), fixed order.
 //   Budget: 1024 + 2048 + ~2600 = ~5700 slots -> ~72 % (STAT), ~62 % streamed.
-// Barriers: TMA bytes (own + multicast from the partner CTA) are credited to every CTA's OWN full barrier; the non-leader
-// CTA of a pair relays "my operands have landed" to its leader (mbarrier remote arrive), which issues the MMAs; stage
-// release (tcgen05.commit) is multicast to all four CTAs because a stage is written by two of them.
+// Barriers: the two pairs load independently.  Both CTAs of a pair credit their TMA bytes to the leader's full barrier (the
+// dx2 kernel's producer), the leader issues the MMAs and its tcgen05.commit releases the stage in both CTAs of the pair;
+// the pairs of a cluster meet only in the radial-dot exchange.  (Sharing the P tile between the pairs by multicast coupled
+// them through the stage barriers and measured slower: profiles/README.md r02.)
 // ================================================================================================
 struct Dw4Params {
   int n_rows, n_classes;
@@ -1524,16 +1480,12 @@ struct Dw4Params {
   float* dw;                     // [n_classes, 512]
   int accumulate;
   long long* dbg;
-  int exp;                       // timing experiments only (FEDFR_DW_EXP, wrong results): 1 no w_hat loads, 2 no dw stores, 4 no lane reduction
 };
 constexpr int kDw4EpiWarps = 16;                 // warp (quad, cgp): e rows [32 quad, +32) of this CTA, classes [64 cgp, +64) of the item
 constexpr int kDw4Threads = (kDw4EpiWarps + 2) * 32;
 constexpr int kDw4E = 512;
 
-// LITE: no cross-pair multicast and no relay -- every CTA loads the whole P tile of its class tile itself and the TMA bytes
-// of both CTAs of a pair are credited straight to the leader's full barrier (the dx2 kernel's producer); the two pairs of a
-// cluster then only meet in the radial-dot exchange.  16 KB more from L2 per CTA and k-block, no coupling between the pairs.
-template <bool STAT, int STAGES, bool LITE = false>
+template <bool STAT, int STAGES>
 __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_constant__ CUtensorMap tmap_x,
                                                              const Dw4Params p) {
   extern __shared__ uint8_t smem_raw[];
@@ -1548,33 +1500,29 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
   float* tsum = part + 4 * 256;                                                // [2][4 CTAs][256]            per-CTA sums, all CTAs
   float2* scal = reinterpret_cast<float2*>(tsum + 2 * 4 * 256);                // [256]                       (1/n_j, -t_j/n_j)
   uint64_t* bars = reinterpret_cast<uint64_t*>(scal + 256);
-  uint64_t* full = bars;                          // [STAGES]  own + multicast bytes of this CTA's stage
-  uint64_t* empty = bars + STAGES;                // [STAGES]  2 arrivals: the commit of each pair's leader
-  uint64_t* peer_full = bars + 2 * STAGES;        // [STAGES]  leader only: the other CTA of the pair has its stage
-  uint64_t* tmem_full = bars + 3 * STAGES;        // [2]
-  uint64_t* tmem_empty = bars + 3 * STAGES + 2;   // [2]       leader only: epilogue warps of both CTAs
-  uint64_t* tbar = bars + 3 * STAGES + 4;         // [2]       per-CTA sums of all four CTAs have landed
-  uint64_t* x_full = bars + 3 * STAGES + 6;
-  uint64_t* peer_x_full = bars + 3 * STAGES + 7;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * STAGES + 8);
+  uint64_t* full = bars;                          // [STAGES]  leader only: stage bytes of both CTAs of the pair
+  uint64_t* empty = bars + STAGES;                // [STAGES]  the commit of the pair's leader
+  uint64_t* tmem_full = bars + 2 * STAGES;        // [2]
+  uint64_t* tmem_empty = bars + 2 * STAGES + 2;   // [2]       leader only: epilogue warps of both CTAs
+  uint64_t* tbar = bars + 2 * STAGES + 4;         // [2]       per-CTA sums of all four CTAs have landed
+  uint64_t* x_full = bars + 2 * STAGES + 6;       // STAT, leader only: the resident x_scaled^T of both CTAs of the pair
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 7);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t crank = cluster_ctarank();
   const int hs = (int)(crank >> 1), cpar = (int)(crank & 1);      // e-slice of the pair; N-half (class tile parity) inside the pair
   const bool leader = cpar == 0;
-  const uint32_t leader_rank = crank & ~1u, partner = crank ^ 2u;  // partner: same class tile, other e-slice
+  const uint32_t leader_rank = crank & ~1u;
   const int n_clusters = gridDim.x >> 2, cid = blockIdx.x >> 2;
   const int n_kb = (p.n_rows + BK - 1) / BK;
   constexpr int kProducerWarp = kDw4EpiWarps, kMmaWarp = kDw4EpiWarps + 1;
   const uint16_t pair_mask = (uint16_t)(3u << (2 * hs));
-  const uint16_t p_mask = (uint16_t)((1u << cpar) | (1u << (cpar + 2)));
   const int e_cta = hs * 256 + cpar * 128;                        // first e of this CTA's 128 M rows
 
   if (threadIdx.x == 0) {
-    for (int i = 0; i < STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], LITE ? 1 : 2); mbar_init(&peer_full[i], 1); }
+    for (int i = 0; i < STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 2 * kDw4EpiWarps); mbar_init(&tbar[i], 4 * 8); }
     mbar_init(x_full, 1);
-    mbar_init(peer_x_full, 1);
     fence_barrier_init();
   }
   if (warp == kProducerWarp && lane == 0) { prefetch_tmap(&tmap_g); prefetch_tmap(&tmap_x); }
@@ -1588,14 +1536,10 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
     if (lane == 0) {
       const uint32_t x_full_leader = mapa_u32(smem_u32(x_full), leader_rank);
       if (STAT) {
-        if (LITE) { if (leader) mbar_arrive_expect_tx(x_full, 2 * n_kb * kXBytes); }
-        else mbar_arrive_expect_tx(x_full, n_kb * kXBytes);
+        if (leader) mbar_arrive_expect_tx(x_full, 2 * n_kb * kXBytes);
         for (int kb = 0; kb < n_kb; ++kb)
 #pragma unroll
-          for (int nb = 0; nb < 2; ++nb) {
-            if (LITE) tma_load_2d_2cta(smem_x + kb * kXBytes + nb * kBoxBytes, &tmap_x, x_full_leader, e_cta + nb * 64, kb * BK);
-            else tma_load_2d(smem_x + kb * kXBytes + nb * kBoxBytes, &tmap_x, x_full, e_cta + nb * 64, kb * BK);
-          }
+          for (int nb = 0; nb < 2; ++nb) tma_load_2d_2cta(smem_x + kb * kXBytes + nb * kBoxBytes, &tmap_x, x_full_leader, e_cta + nb * 64, kb * BK);
       }
       PipeState ps;
       for (int i = 0; i * n_clusters + cid < p.n_tp; ++i) {
@@ -1603,24 +1547,14 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
         for (int kb = 0; kb < n_kb; ++kb) {
           mbar_wait_cluster(&empty[ps.stage], ps.phase ^ 1);
           uint8_t* sp = smem_st + ps.stage * kStageBytes;
-          if (LITE) {
-            const uint32_t full_leader = mapa_u32(smem_u32(&full[ps.stage]), leader_rank);
-            if (leader) mbar_arrive_expect_tx(&full[ps.stage], 2 * kStageBytes);
+          const uint32_t full_leader = mapa_u32(smem_u32(&full[ps.stage]), leader_rank);
+          if (leader) mbar_arrive_expect_tx(&full[ps.stage], 2 * kStageBytes);
 #pragma unroll
-            for (int hb = 0; hb < 2; ++hb)
-              tma_load_2d_2cta(sp + hb * kBoxBytes, &tmap_g, full_leader, 0, ((2 * ct + hb) * p.n_rb + (kb >> 1)) * BM + (kb & 1) * 64);
-            if (!STAT) {
+          for (int hb = 0; hb < 2; ++hb)
+            tma_load_2d_2cta(sp + hb * kBoxBytes, &tmap_g, full_leader, 0, ((2 * ct + hb) * p.n_rb + (kb >> 1)) * BM + (kb & 1) * 64);
+          if (!STAT) {
 #pragma unroll
-              for (int nb = 0; nb < 2; ++nb) tma_load_2d_2cta(sp + kPBytes + nb * kBoxBytes, &tmap_x, full_leader, e_cta + nb * 64, kb * BK);
-            }
-          } else {
-            mbar_arrive_expect_tx(&full[ps.stage], kStageBytes);
-            // 64-class box `hs` of the P tile, for this CTA and its partner in the other pair
-            tma_load_2d_mc(sp + hs * kBoxBytes, &tmap_g, &full[ps.stage], 0, ((2 * ct + hs) * p.n_rb + (kb >> 1)) * BM + (kb & 1) * 64, p_mask);
-            if (!STAT) {
-#pragma unroll
-              for (int nb = 0; nb < 2; ++nb) tma_load_2d(sp + kPBytes + nb * kBoxBytes, &tmap_x, &full[ps.stage], e_cta + nb * 64, kb * BK);
-            }
+            for (int nb = 0; nb < 2; ++nb) tma_load_2d_2cta(sp + kPBytes + nb * kBoxBytes, &tmap_x, full_leader, e_cta + nb * 64, kb * BK);
           }
           ps.advance(STAGES);
         }
@@ -1631,7 +1565,7 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
       constexpr uint32_t idesc = make_idesc_bf16(2 * BM, 256, true, true);
       PipeState ps;
       long long t_we = 0, t_wf = 0, t_all = clock64();
-      if (STAT) { mbar_wait_cluster(x_full, 0); if (!LITE) mbar_wait_cluster(peer_x_full, 0); }
+      if (STAT) mbar_wait_cluster(x_full, 0);
       for (int it = 0; it * n_clusters + cid < p.n_tp; ++it) {
         const int acc = it & 1;
         long long c0 = clock64();
@@ -1641,8 +1575,7 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
         const uint32_t d_tmem = tmem_base + acc * 256;
         for (int kb = 0; kb < n_kb; ++kb) {
           c0 = clock64();
-          if (LITE) mbar_wait_cluster(&full[ps.stage], ps.phase);
-          else { mbar_wait(&full[ps.stage], ps.phase); mbar_wait_cluster(&peer_full[ps.stage], ps.phase); }
+          mbar_wait_cluster(&full[ps.stage], ps.phase);
           t_wf += clock64() - c0;
           tc_fence_after();
           const uint32_t p_addr = smem_u32(smem_st + ps.stage * kStageBytes);
@@ -1653,22 +1586,12 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
             const uint64_t db = make_desc_sw128(p_addr + kk * 2048, kBoxBytes, 1024);     // B = P           (N = classes, MN-major)
             umma_bf16_ss_2cta(d_tmem, da, db, idesc, (kb | kk) != 0);
           }
-          umma_commit_2cta(&empty[ps.stage], LITE ? pair_mask : (uint16_t)0xF);          // (not LITE: the stage is written by CTAs of both pairs)
+          umma_commit_2cta(&empty[ps.stage], pair_mask);
           ps.advance(STAGES);
         }
         umma_commit_2cta(&tmem_full[acc], pair_mask);
       }
       if (p.dbg && blockIdx.x == 0) { p.dbg[0] = t_we; p.dbg[1] = t_wf; p.dbg[2] = clock64() - t_all; }
-    } else if (lane == 0 && !LITE) {
-      // relay: tell the leader of this pair when this CTA's operands of a stage have landed
-      PipeState ps;
-      if (STAT) { mbar_wait(x_full, 0); mbar_arrive_remote(peer_x_full, leader_rank); }
-      for (int it = 0; it * n_clusters + cid < p.n_tp; ++it)
-        for (int kb = 0; kb < n_kb; ++kb) {
-          mbar_wait(&full[ps.stage], ps.phase);
-          mbar_arrive_remote(&peer_full[ps.stage], leader_rank);
-          ps.advance(STAGES);
-        }
     }
   } else {
     // ------------------------------------------------------------------ epilogue: thread = e row, register = class
@@ -1688,10 +1611,7 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
       uint32_t wpk[32];
       const int n_ok = p.n_classes - cls_w;                 // classes of this group that exist (>= 64 for all but the last tiles)
       const unsigned short* wt = wbase + (int64_t)cls_w * kDw4E;
-      if (p.exp & 1) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) wpk[j] = 0x3f803f80u;
-      } else if (n_ok >= 64) {
+      if (n_ok >= 64) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) wpk[j] = (uint32_t)__ldg(wt + (2 * j) * kDw4E) | ((uint32_t)__ldg(wt + (2 * j + 1) * kDw4E) << 16);
       } else {
@@ -1721,7 +1641,7 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
           v[j] = __float_as_uint(pr.x);
           v[j + 1] = __float_as_uint(pr.y);
         }
-        part[quad * 256 + cgp * 64 + c * 32 + lane] = (p.exp & 4) ? __uint_as_float(v[0]) : warp_colsum32_bits(v, lane);
+        part[quad * 256 + cgp * 64 + c * 32 + lane] = warp_colsum32_bits(v, lane);
       }
       t_p1 += clock() - c0;
       c0 = clock();
@@ -1755,7 +1675,7 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
       t_ex += clock() - c0;
       c0 = clock();
       // ---- pass 2: dw[class][e] = acc / n - w_hat (t / n): one full 128-byte line per warp and class, straight from registers
-      const bool plain = n_ok >= 64 && !p.accumulate && !(p.exp & 2);      // the common case: no per-class predicates at all
+      const bool plain = n_ok >= 64 && !p.accumulate;      // the common case: no per-class predicates at all
 #pragma unroll
       for (int c = 0; c < 2; ++c) {
         uint32_t v[32];
@@ -1781,7 +1701,6 @@ __global__ void __launch_bounds__(kDw4Threads, 1) dw4_kernel(const __grid_consta
             float2 r = __ffma2_rn(make_float2(__uint_as_float(w2 << 16), __uint_as_float(w2 & 0xffff0000u)), make_float2(sc.y, sc.w),
                                   __fmul2_rn(make_float2(__uint_as_float(v[j]), __uint_as_float(v[j + 1])), make_float2(sc.x, sc.z)));
             float* d = out + j * kDw4E;
-            if (p.exp & 2) { if (r.x == 1.2345f && r.y == 5.4321f) d[0] = r.x; continue; }
             if (p.accumulate) {
               if (c * 32 + j < n_ok) r.x += d[0];
               if (c * 32 + j + 1 < n_ok) r.y += d[kDw4E];
@@ -2012,7 +1931,6 @@ static BwdPlan make_bwd_plan(int64_t n_rows, int64_t n_classes, int emb) {
   const int64_t c_pad = (n_classes + 255) / 256 * 256;
   const int64_t row_bytes = n_rb * BM * 2;           // bytes of G scratch per class
   int64_t budget_seq = 512ll << 20, budget_pipe = 32ll << 20;
-  if (const char* e = getenv("FEDFR_G_CHUNK_MB")) { long v = atol(e); if (v > 0) budget_seq = budget_pipe = (int64_t)v << 20; }
   if (g_chunk_budget_mb > 0) budget_seq = budget_pipe = g_chunk_budget_mb << 20;
   auto chunk_for = [&](int64_t budget) {
     int64_t c = budget / row_bytes / 256 * 256;
@@ -2121,33 +2039,20 @@ static int launch_dx(const CUtensorMap& tg, const CUtensorMap& tw, const DxParam
   return launch_dx_cs<BN, 1>(tg, tw, p, grid, st);
 }
 
-template <int EMB, int CS, bool P2 = false, int EW = kDwEpiWarps>
+template <int EMB, int CS>
 static int launch_dw_cs(const CUtensorMap& tg, const CUtensorMap& tx, const CUtensorMap& twh, const CUtensorMap& tdw, const DwParams& p, int grid,
                         cudaStream_t st) {
   constexpr int EN = EMB < 256 ? EMB : 256;
-  constexpr int kStage = 2 * kBoxBytes + (P2 ? 2 : EN / 64) * kBoxBytes;
-  constexpr int NG = EN / (EW / 4) / 32;                         // 32-column groups per epilogue warp
-  constexpr int kEpi = EW * ((NG + 1) / 2) * 4096 + (NG == 1 ? EW * 2 * 4096 : ((P2 && NG == 4) ? EW * 4096 : 0));   // w_hat boxes (= staging) [+ staging]
+  constexpr int kStage = 2 * kBoxBytes + (EN / 64) * kBoxBytes;
+  constexpr int NG = EN / (kDwEpiWarps / 4) / 32;                // 32-column groups per epilogue warp
+  constexpr int kEpi = kDwEpiWarps * ((NG + 1) / 2) * 4096 + (NG == 1 ? kDwEpiWarps * 2 * 4096 : 0);   // w_hat boxes (= staging) [+ staging]
   constexpr int kFixed = 8192 /* partial dots */ + 1024 /* alignment */ + 512 /* barriers */;
   constexpr int STAGES = (232448 - kFixed - kEpi) / kStage > 8 ? 8 : (232448 - kFixed - kEpi) / kStage;
   static_assert(STAGES >= 2, "dw kernel smem budget");
   const size_t smem = (size_t)STAGES * kStage + kEpi + kFixed;
-  return launch_cluster_threads(dw_kernel<EMB, STAGES, CS, P2, EW>, (EW + 2) * 32, grid, CS, smem, st, tg, tx, twh, tdw, p);
+  return launch_cluster_threads(dw_kernel<EMB, STAGES, CS>, kDwThreads, grid, CS, smem, st, tg, tx, twh, tdw, p);
 }
 
-static int g_dw_p2 = getenv("FEDFR_DW_P2") ? atoi(getenv("FEDFR_DW_P2")) : 0;      // 1: the pair kernel on cta_group::2 pairs (clusters of 4) for E = 512
-// E = 512, cta_group::2 pairs: clusters of four CTAs, each taking two class tiles per item
-static int launch_dw_p2(const CUtensorMap& tg, const CUtensorMap& tx, const CUtensorMap& twh, const CUtensorMap& tdw, const DwParams& p, int n_ct,
-                        int sms, cudaStream_t st) {
-  const int n_groups = (n_ct + 1) / 2;
-  int clusters = sms / 4 * 9 / 10;                       // GPC packing of 4-CTA clusters leaves a few SMs unused
-  if (clusters > sms / 4) clusters = sms / 4;
-  if (clusters > n_groups) clusters = n_groups;
-  if (clusters < 1) clusters = 1;
-  return launch_dw_cs<512, 4, true>(tg, tx, twh, tdw, p, clusters * 4, st);
-}
-
-static int g_dw_ew = getenv("FEDFR_DW_EW") ? atoi(getenv("FEDFR_DW_EW")) : 8;      // epilogue warps of the E = 512 pair kernel (8 or 16)
 template <int EMB>
 static int launch_dw(const CUtensorMap& tg, const CUtensorMap& tx, const CUtensorMap& twh, const CUtensorMap& tdw, const DwParams& p, int n_ct,
                      int cs, int sms, cudaStream_t st) {
@@ -2161,7 +2066,6 @@ static int launch_dw(const CUtensorMap& tg, const CUtensorMap& tx, const CUtenso
   const int clusters = n_groups < max_clusters ? n_groups : max_clusters;
   const int grid = clusters * cs;
   if constexpr (EMB > 256) {
-    if (g_dw_ew == 16) return launch_dw_cs<EMB, 2, false, 16>(tg, tx, twh, tdw, p, grid, st);
     return launch_dw_cs<EMB, 2>(tg, tx, twh, tdw, p, grid, st);
   } else {
     if constexpr (EMB >= 128) {
@@ -2172,15 +2076,14 @@ static int launch_dw(const CUtensorMap& tg, const CUtensorMap& tx, const CUtenso
   }
 }
 
-// dw kernel choice for E = 512 (pfc_set_dw4 / FEDFR_DW4):  -1 (default) automatic: the 4-CTA-cluster transposed kernel with
-// independent pairs (LITE) from 2048 gathered rows on -- there its shared-memory-pipe savings in the mainloop win (measured
-// r02i: 0.72 vs 0.85 ms at Bt = 4096) --, the e-split pair kernel below that, where dw4's longer epilogue chain is not yet
-// amortised by the K loop (1.73 vs 1.02 ms at Bt = 512);  0: never;  1: dw4 with cross-pair multicast;  2: dw4 LITE always.
-static int g_dw4 = getenv("FEDFR_DW4") ? atoi(getenv("FEDFR_DW4")) : -1;
-static int dw4_mode(int64_t n_rows, int emb) {       // 0 = pair kernel, 1 = multicast, 2 = LITE
-  if (emb != 512 || g_dw4 == 0) return 0;
-  if (g_dw4 < 0) return n_rows >= 2048 ? 2 : 0;
-  return g_dw4;
+// dw kernel choice for E = 512 (pfc_set_dw4):  -1 (default) automatic: the 4-CTA-cluster transposed kernel from 2048
+// gathered rows on -- there its shared-memory-pipe savings in the mainloop win (measured r02i: 0.72 vs 0.85 ms at
+// Bt = 4096) --, the e-split pair kernel below that, where dw4's longer epilogue chain is not yet amortised by the K loop
+// (1.73 vs 1.02 ms at Bt = 512);  0: never;  1: always.
+static int g_dw4 = -1;
+static bool dw4_chosen(int64_t n_rows, int emb) {
+  if (emb != 512 || g_dw4 == 0) return false;
+  return g_dw4 > 0 || n_rows >= 2048;
 }
 template <bool STAT, int STAGES>
 static size_t dw4_smem_bytes() {
@@ -2223,10 +2126,6 @@ static int launch_dw4(const CUtensorMap& tg, const CUtensorMap& tx, const Dw4Par
   if (clusters > cap) clusters = cap;
   if (clusters > p.n_tp) clusters = p.n_tp;
   if (clusters < 1) clusters = 1;
-  if (dw4_mode(p.n_rows, 512) == 2) {      // LITE: independent pairs (no cross-pair multicast, no relay)
-    if (stat) return launch_cluster_threads(dw4_kernel<true, kDw4StagesStat, true>, kDw4Threads, clusters * 4, 4, dw4_smem_bytes<true, kDw4StagesStat>(), st, tg, tx, p);
-    return launch_cluster_threads(dw4_kernel<false, kDw4StagesStream, true>, kDw4Threads, clusters * 4, 4, dw4_smem_bytes<false, kDw4StagesStream>(), st, tg, tx, p);
-  }
   if (stat) return launch_cluster_threads(dw4_kernel<true, kDw4StagesStat>, kDw4Threads, clusters * 4, 4, dw4_smem_bytes<true, kDw4StagesStat>(), st, tg, tx, p);
   return launch_cluster_threads(dw4_kernel<false, kDw4StagesStream>, kDw4Threads, clusters * 4, 4, dw4_smem_bytes<false, kDw4StagesStream>(), st, tg, tx, p);
 }
@@ -2558,16 +2457,11 @@ static int tc_normalize_fwd_enqueue(const float* w, const int64_t* index, const 
     p.n_rb = (int)((n_rows + BM - 1) / BM); p.n_ct = (int)((cc + bn - 1) / bn);
     p.s = s; p.m = m; p.margin_kind = margin_kind; p.part_max = part_max; p.part_sum = part_sum; p.target_logit = target_logit; p.accumulate_stats = k > 0; p.prefetch = g_prefetch[0];
     p.row_bound = row_bound; p.target_cos = target_cos; p.ldg = L.c_pad;
-    static const int fwd_exp = getenv("FEDFR_FWD_EXP") ? atoi(getenv("FEDFR_FWD_EXP")) : 0;
-    p.exp = fwd_exp;
     if (has_next) {
       p.norm_w = index ? w : w + n0 * emb; p.norm_index = index ? index + n0 : nullptr; p.norm_rows = chunk_len(n0);
       p.norm_out = wh + n0 * emb; p.norm_inv = inv_norm + n0;
     }
     const int grid = g_logits_pair ? pair_grid(n_rows, cc) : fwd_grid(n_rows, cc, bn);
-    static const int exp_mode = getenv("FEDFR_EXP") ? atoi(getenv("FEDFR_EXP")) : 0;      // timing experiments only (wrong results)
-    if (exp_mode == 1) p.norm_rows = 0;          // big CTA, idle normaliser warps
-    if (exp_mode == 2) p.n_ct = 0;               // normaliser warps only
     prof_begin(PH_FWD, st);
     int rc;
     if (!g_logits_pair) rc = dispatch_logits<MODE_STATS>(tx, tw, p, bn, grid, st);
@@ -2638,7 +2532,7 @@ static ProbBwdPlan make_prob_bwd_plan(int64_t n_rows, int64_t n_classes, int emb
   // dx and dw run side by side on disjoint SMs; pick the k-split whose slower side finishes first
   int64_t best = 0;
   float best_t = 0.f;
-  const float dw_rate = dw4_mode(n_rows, emb) ? g_prob_dw4_rate : g_prob_dw_rate;
+  const float dw_rate = dw4_chosen(n_rows, emb) ? g_prob_dw4_rate : g_prob_dw_rate;
   for (int64_t ks = 1; ks <= max_ks && units * ks <= sms - 16; ++ks) {
     const float t_dx = 1.f / (float)(units * ks), t_dw = 1.f / (dw_rate * (float)(sms - units * ks));
     const float t = g_prob_dx_sms > 0 ? fabsf((float)(units * ks - g_prob_dx_sms)) : (t_dx > t_dw ? t_dx : t_dw);
@@ -2713,12 +2607,10 @@ static int tc_bwd_prob_enqueue(const void* w_hat, const float* inv_norm, const i
   if (paced) dp.sweep = SweepSync{sweep_ctr, sweep_ctr + 1, g_sweep_lead};
   dp.n_rows = (int)n_rows; dp.n_classes = (int)n_classes; dp.emb = emb; dp.n_rb = n_rb; dp.n_eh = pl.n_eh; dp.ksplit = pl.ksplit;
   dp.dx_part = dx_part; dp.accumulate = 0; dp.prefetch = g_prefetch[1]; dp.strided = pl.side_by_side ? 1 : 0;
-  static const int exp_mode = getenv("FEDFR_EXP") ? atoi(getenv("FEDFR_EXP")) : 0;      // timing experiments only (wrong results)
   auto enqueue_dx = [&]() -> int {
     int rc = 0;
     prof_begin(PH_DX, sX);
-    if (exp_mode == 3) rc = 0;                   // dw alone
-    else if (pl.dx_pair) rc = launch_dx2(tg_k, tw_mn, dp, pl.dx_ctas, sX);
+    if (pl.dx_pair) rc = launch_dx2(tg_k, tw_mn, dp, pl.dx_ctas, sX);
     else switch (pl.dx_bn) {
       case 256: rc = launch_dx<256>(tg_k, tw_mn, dp, pl.dx_ctas, pl.dcs, sX); break;
       case 128: rc = launch_dx<128>(tg_k, tw_mn, dp, pl.dx_ctas, pl.dcs, sX); break;
@@ -2728,25 +2620,21 @@ static int tc_bwd_prob_enqueue(const void* w_hat, const float* inv_norm, const i
     prof_end(PH_DX, sX);
     return 0;
   };
-  const bool use_dw4 = dw4_mode(n_rows, emb) != 0;
+  const bool use_dw4 = dw4_chosen(n_rows, emb);
   auto enqueue_dw = [&]() -> int {
     int rc = 0;
     DwParams wp{};
     if (paced) wp.sweep = SweepSync{sweep_ctr + 1, sweep_ctr, g_sweep_lead};
     wp.n_rows = (int)n_rows; wp.n_classes = (int)n_classes; wp.emb = emb; wp.n_ct = (int)((n_classes + BM - 1) / BM); wp.n_rb = n_rb;
     wp.inv_norm = inv_norm; wp.accumulate = accumulate_dw; wp.dbg = g_dbg; wp.prefetch = g_prefetch[2];
-    static const int dw_exp = getenv("FEDFR_DW_EXP") ? atoi(getenv("FEDFR_DW_EXP")) : 0;
-    wp.exp = dw_exp;
     prof_begin(PH_DW, sW);
-    if (exp_mode == 4) rc = 0;                   // dx alone
-    else if (use_dw4) {
+    if (use_dw4) {
       Dw4Params qp{};
       qp.n_rows = (int)n_rows; qp.n_classes = (int)n_classes; qp.n_rb = n_rb; qp.n_tp = (int)((n_classes + 255) / 256);
-      qp.inv_norm = inv_norm; qp.w_hat = wh; qp.dw = dw; qp.accumulate = accumulate_dw; qp.dbg = g_dbg; qp.exp = dw_exp;
+      qp.inv_norm = inv_norm; qp.w_hat = wh; qp.dw = dw; qp.accumulate = accumulate_dw; qp.dbg = g_dbg;
       rc = launch_dw4(tg_mn, tx_mn, qp, pl.sm_dw, sW);
     } else switch (emb) {
-      case 512: rc = g_dw_p2 ? launch_dw_p2(tg_mn, tx_mn, twh_e, tdw_e, wp, wp.n_ct, pl.sm_dw, sW)
-                             : launch_dw<512>(tg_mn, tx_mn, twh_e, tdw_e, wp, wp.n_ct, g_dw_cluster, pl.sm_dw, sW); break;
+      case 512: rc = launch_dw<512>(tg_mn, tx_mn, twh_e, tdw_e, wp, wp.n_ct, g_dw_cluster, pl.sm_dw, sW); break;
       case 256: rc = launch_dw<256>(tg_mn, tx_mn, twh_e, tdw_e, wp, wp.n_ct, g_dw_cluster, pl.sm_dw, sW); break;
       case 128: rc = launch_dw<128>(tg_mn, tx_mn, twh_e, tdw_e, wp, wp.n_ct, g_dw_cluster, pl.sm_dw, sW); break;
       default: rc = launch_dw<64>(tg_mn, tx_mn, twh_e, tdw_e, wp, wp.n_ct, g_dw_cluster, pl.sm_dw, sW); break;
@@ -2790,7 +2678,7 @@ int tc_bwd_prob(const void* x, const void* w_hat, const float* inv_norm, const i
   kb.add(4).add(x).add(w_hat).add(inv_norm).add(label).add(row_sum).add(dx).add(dw).add(workspace).add(prob_ws).add(n_rows).add(n_classes)
       .add(workspace_bytes).add(emb).add(accumulate_dw).add(s).add(m).add(margin_kind).add(inv_total_batch).add(g_logits_pair).add(g_dx_cluster)
       .add(g_dw_cluster).add(g_prob_dx_sms).add(g_prob_dw_rate).add(g_sweep_lead).add(g_prefetch[1]).add(g_prefetch[2]).add(g_dx_pair)
-      .add(range_flag_of_current_device()).add(g_dw4).add(g_dw_p2).add(g_dw_ew);
+      .add(range_flag_of_current_device()).add(g_dw4);
   if (kb.overflow) return enqueue(st);
   return run_cached_graph(kb, st, enqueue);
 }
@@ -2894,7 +2782,7 @@ int tc_set_range_flag(int* flag, float limit_nats) {
   return 0;
 }
 void tc_set_graph(int on) { g_use_graph = on ? 1 : 0; }
-void tc_set_dw4(int on) { g_dw4 = on < 0 ? -1 : (on > 2 ? 2 : on); }
+void tc_set_dw4(int on) { g_dw4 = on < 0 ? -1 : (on > 0 ? 1 : 0); }
 void tc_set_dx_pair(int on) { g_dx_pair = on ? 1 : 0; }
 void tc_set_prefetch(int logits, int dx, int dw) { g_prefetch[0] = logits; g_prefetch[1] = dx; g_prefetch[2] = dw; }
 void tc_set_pipeline(int on, int sm_g, int sm_dx, int sm_dw, int ring) {

@@ -31,8 +31,8 @@ int pfc_set_logits_pair(int on);                            /* [1] cta_group::2 
 int pfc_set_logits_tile(int bn);                            /* [128] class-tile width of the single-CTA logits kernels (128 / 256) */
 int pfc_set_dx_pair(int on);                                /* [1] cta_group::2 dx kernel when ceil(Bt / 128) % 4 == 0, E >= 256 and
                                                                pfc_set_logits_pair is on (the last row block may be partial) */
-int pfc_set_dw4(int mode);                                  /* [FEDFR_DW4 or -1] E = 512 dw kernel: -1 auto (4-CTA-cluster kernel from 2048 gathered rows on),
-                                                               0 e-split pair kernel, 1 cluster kernel with cross-pair multicast, 2 cluster kernel, independent pairs */
+int pfc_set_dw4(int mode);                                  /* [-1] E = 512 dw kernel: -1 auto (4-CTA-cluster kernel from 2048 gathered rows on),
+                                                               0 e-split pair kernel, > 0 4-CTA-cluster kernel */
 int pfc_set_clusters(int dx_cluster, int dw_cluster);       /* [2, 2] cluster sizes of the single-CTA dx / dw kernels (1, 2, 4) */
 int pfc_set_fwd_overlap(int chunks, int norm_blocks_per_sm);/* [4, 2] class chunks of the fused forward; normalise blocks per SM */
 int pfc_set_prefetch(int logits, int dx_distance, int dw);  /* [0, 0, 0] TMA L2 prefetch ahead of the shared-memory rings */

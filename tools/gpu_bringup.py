@@ -241,11 +241,13 @@ def stage_bwd_tc():
 
 
 def stage_bwd_tc_big():
-    import os
     from fedfr_b200 import _native as N
-    os.environ["FEDFR_G_CHUNK_MB"] = "16"      # force several chunks
-    print("tensor path B=512 C=40000 E=512 (multi-chunk)", flush=True)
-    _check_fwd_bwd(N.PATH_TENSOR, 512, 40000, 512)
+    N.lib.pfc_set_chunk_mb(16)                 # force several chunks
+    try:
+        print("tensor path B=512 C=40000 E=512 (multi-chunk)", flush=True)
+        _check_fwd_bwd(N.PATH_TENSOR, 512, 40000, 512)
+    finally:
+        N.lib.pfc_set_chunk_mb(0)
 
 
 def stage_step_tc():
