@@ -62,6 +62,8 @@ SIGNATURES = {
     "pfc_pair_scores": (_i32, [_vp, _i64, _i32, _vp, _vp, _i64, _vp, _vp]),
     "pfc_tar_at_far_workspace_bytes": (_sz, [_i64]),
     "pfc_tar_at_far": (_i32, [_vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _sz, _vp]),
+    "pfc_roc_curve_workspace_bytes": (_sz, [_i64]),
+    "pfc_roc_curve": (_i32, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "fedavg_table_bytes": (_sz, [_i32, _i32]),
     "fedavg_weighted_sum": (_i32, [_vp, _vp, _vp, _vp, _i32, _vp, _i32, _vp, _sz, _vp]),
     "fedavg_blend": (_i32, [_vp, _vp, _f32, _f32, _i64, _vp, _vp]),

@@ -18,6 +18,13 @@
 // selections with the same key prefix share one histogram (prefixes of one length are equal or disjoint, so each key
 // lands in at most one), counted with warp-aggregated shared atomics; the last block to finish a pass picks the bins.
 // One counting pass then accepts score > threshold for every FAR.  No sort of the scores.
+//
+// ROC curve (sklearn.metrics.roc_curve with drop_intermediate): the TAR keys, complemented so that ascending order is
+// descending score, are sorted with a stable 4 x 8-bit LSD radix sort that carries the class byte (per pass: a tile
+// histogram, a scan of each digit's row over the tiles, a scatter ranked with match.any).  Reduce-then-scan passes over
+// the sorted keys then cut it into runs of one key (tps = genuine up to the run's end, fps = its position + 1 - tps),
+// apply sklearn's thinning stencil to the runs and compact the kept points in order.  Integer counts and scans only: the
+// result does not depend on the schedule.
 #include "common.cuh"
 #include "../../fedfr_b200/csrc/dot_chain.cuh"
 
@@ -312,6 +319,361 @@ __global__ void tar_finish_kernel(const TarState* st, int n_far, int64_t* counts
   }
 }
 
+constexpr int kRocThreads = 256;               // every ROC kernel runs 256 threads: one per digit where it works on digits
+constexpr int kRocItems = 8;
+constexpr int kRocTile = kRocThreads * kRocItems;
+constexpr int kRocWarps = kRocThreads / 32;
+constexpr int kRocColTiles = 32;               // tiles per block of the digit-offset scan
+
+struct RocState {
+  unsigned long long n_gen, n_imp, n_bad;      // finite genuine, finite impostor, NaN or +-inf scores
+  unsigned int run_totals[2];                  // distinct keys (runs), genuine pairs (from the run scan)
+  unsigned int n_keep;                         // runs kept by the thinning
+};
+
+// Sort key: tar_key complemented, so that ascending keys are descending scores.  Counts and positions fit 32 bits: n < 2^31.
+__device__ __forceinline__ unsigned int roc_sort_key(unsigned int u) { return ~tar_key(u); }
+
+__device__ __forceinline__ double roc_key_value(unsigned int sort_key) {
+  const unsigned int key = ~sort_key;
+  union { unsigned int u; float f; } v;
+  v.u = (key & 0x80000000u) ? (key & 0x7fffffffu) : ~key;
+  return (double)v.f;
+}
+
+// Exclusive prefix sum of v over the block's threads (blockDim = kRocThreads); the block's sum -> *total.
+__device__ unsigned int roc_block_scan(unsigned int v, unsigned int* total) {
+  __shared__ unsigned int warp_tot[kRocWarps];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  unsigned int x = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned int y = __shfl_sync(0xffffffffu, x, lane >= o ? lane - o : lane);
+    if (lane >= o) x += y;
+  }
+  if (lane == 31) warp_tot[w] = x;
+  __syncthreads();
+  unsigned int before = 0, all = 0;
+  for (int i = 0; i < kRocWarps; ++i) {
+    before += i < w ? warp_tot[i] : 0u;
+    all += warp_tot[i];
+  }
+  __syncthreads();                             // warp_tot is rewritten by the next call
+  *total = all;
+  return before + x - v;
+}
+
+// One sort pass, step 1: hist[tile][digit] = count of `digit` at bit `shift` in this tile.  The first pass reads the scores
+// (bits, issame) and counts the classes; later passes read the previous pass's keys.
+__global__ void __launch_bounds__(kRocThreads)
+roc_hist_kernel(const unsigned int* __restrict__ bits, const unsigned char* __restrict__ issame,
+                const unsigned int* __restrict__ keys, int64_t n, int shift, unsigned int* __restrict__ hist, RocState* st) {
+  __shared__ unsigned int h[256];
+  const int lane = threadIdx.x & 31;
+  h[threadIdx.x] = 0u;
+  __syncthreads();
+  const int64_t base = (int64_t)blockIdx.x * kRocTile;
+  unsigned int gen = 0, imp = 0, bad = 0;
+  for (int r = 0; r < kRocItems; ++r) {
+    const int64_t i = base + r * kRocThreads + threadIdx.x;
+    unsigned int d = 0x100u + (unsigned int)lane;                      // past the end: a digit of its own, not counted
+    if (i < n) {
+      unsigned int key;
+      if (bits) {
+        const unsigned int u = bits[i];
+        const bool finite = (u & 0x7fffffffu) < 0x7f800000u, g = issame[i] != 0;
+        bad += !finite;
+        gen += finite && g;
+        imp += finite && !g;
+        key = roc_sort_key(u);
+      } else {
+        key = keys[i];
+      }
+      d = (key >> shift) & 0xffu;
+    }
+    const unsigned int peers = __match_any_sync(0xffffffffu, d);
+    if (d < 0x100u && lane == __ffs((int)peers) - 1) atomicAdd(&h[d], (unsigned int)__popc(peers));
+  }
+  if (bits) {                                  // the same for the whole grid
+    unsigned int t;
+    roc_block_scan(gen, &t);
+    if (threadIdx.x == 0) atomicAdd(&st->n_gen, (unsigned long long)t);
+    roc_block_scan(imp, &t);
+    if (threadIdx.x == 0) atomicAdd(&st->n_imp, (unsigned long long)t);
+    roc_block_scan(bad, &t);
+    if (threadIdx.x == 0) atomicAdd(&st->n_bad, (unsigned long long)t);
+  }
+  __syncthreads();
+  hist[(int64_t)blockIdx.x * 256 + threadIdx.x] = h[threadIdx.x];
+}
+
+// Step 2: part[g][digit] = sum of hist[tile][digit] over the kRocColTiles tiles of group g.
+__global__ void __launch_bounds__(kRocThreads)
+roc_col_sum_kernel(const unsigned int* __restrict__ hist, int64_t n_tiles, unsigned int* __restrict__ part) {
+  const int64_t t0 = (int64_t)blockIdx.x * kRocColTiles;
+  const int64_t t1 = t0 + kRocColTiles < n_tiles ? t0 + kRocColTiles : n_tiles;
+  unsigned int s = 0;
+  for (int64_t t = t0; t < t1; ++t) s += hist[t * 256 + threadIdx.x];
+  part[(int64_t)blockIdx.x * 256 + threadIdx.x] = s;
+}
+
+// Step 3 (one block, thread = digit): part[g][digit] = position of group g's first key with that digit in the output.
+__global__ void __launch_bounds__(kRocThreads)
+roc_col_scan_kernel(unsigned int* __restrict__ part, int64_t n_groups) {
+  const int d = threadIdx.x;
+  unsigned int run = 0;
+  for (int64_t g = 0; g < n_groups; ++g) {
+    const unsigned int c = part[g * 256 + d];
+    part[g * 256 + d] = run;
+    run += c;
+  }
+  unsigned int total;
+  const unsigned int digit_base = roc_block_scan(run, &total);
+  for (int64_t g = 0; g < n_groups; ++g) part[g * 256 + d] += digit_base;
+}
+
+// Step 4: hist[tile][digit] = position of the tile's first key with that digit in the output.
+__global__ void __launch_bounds__(kRocThreads)
+roc_col_apply_kernel(unsigned int* __restrict__ hist, int64_t n_tiles, const unsigned int* __restrict__ part) {
+  const int64_t t0 = (int64_t)blockIdx.x * kRocColTiles;
+  const int64_t t1 = t0 + kRocColTiles < n_tiles ? t0 + kRocColTiles : n_tiles;
+  unsigned int run = part[(int64_t)blockIdx.x * 256 + threadIdx.x];
+  for (int64_t t = t0; t < t1; ++t) {
+    const unsigned int c = hist[t * 256 + threadIdx.x];
+    hist[t * 256 + threadIdx.x] = run;
+    run += c;
+  }
+}
+
+// Step 5: stable scatter.  Warp w of a tile owns its keys w * 256 ... w * 256 + 255 in rounds of 32; within a round,
+// lanes with one digit are ranked by match.any and their leader advances the warp's count of that digit.  Tile order is
+// (warp, round, lane) = key order, so equal digits keep their order.
+__global__ void __launch_bounds__(kRocThreads)
+roc_scatter_kernel(const unsigned int* __restrict__ bits, const unsigned char* __restrict__ issame,
+                   const unsigned int* __restrict__ keys_in, const unsigned char* __restrict__ cls_in, int64_t n, int shift,
+                   const unsigned int* __restrict__ hist, unsigned int* __restrict__ keys_out,
+                   unsigned char* __restrict__ cls_out) {
+  __shared__ unsigned int cnt[kRocWarps][256];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  for (int i = threadIdx.x; i < kRocWarps * 256; i += kRocThreads) cnt[i >> 8][i & 255] = 0u;
+  __syncthreads();
+  const int64_t base = (int64_t)blockIdx.x * kRocTile + w * (kRocItems * 32);
+  unsigned int key[kRocItems], rank[kRocItems];
+  unsigned char cls[kRocItems];
+#pragma unroll
+  for (int r = 0; r < kRocItems; ++r) {
+    const int64_t i = base + r * 32 + lane;
+    unsigned int d = 0x100u + (unsigned int)lane;
+    key[r] = 0u;
+    cls[r] = 0;
+    if (i < n) {
+      if (bits) {
+        key[r] = roc_sort_key(bits[i]);
+        cls[r] = issame[i] != 0;
+      } else {
+        key[r] = keys_in[i];
+        cls[r] = cls_in[i];
+      }
+      d = (key[r] >> shift) & 0xffu;
+    }
+    const unsigned int peers = __match_any_sync(0xffffffffu, d);
+    const int leader = __ffs((int)peers) - 1;
+    unsigned int before = 0;
+    if (lane == leader && d < 0x100u) {
+      before = cnt[w][d];
+      cnt[w][d] = before + (unsigned int)__popc(peers);
+    }
+    before = __shfl_sync(0xffffffffu, before, leader);
+    rank[r] = before + (unsigned int)__popc(peers & ((1u << lane) - 1u));
+    __syncwarp();
+  }
+  __syncthreads();
+  {                                            // thread = digit: warp counts -> output positions
+    unsigned int run = hist[(int64_t)blockIdx.x * 256 + threadIdx.x];
+    for (int v = 0; v < kRocWarps; ++v) {
+      const unsigned int c = cnt[v][threadIdx.x];
+      cnt[v][threadIdx.x] = run;
+      run += c;
+    }
+  }
+  __syncthreads();
+#pragma unroll
+  for (int r = 0; r < kRocItems; ++r) {
+    if (base + r * 32 + lane < n) {
+      const unsigned int dst = cnt[w][(key[r] >> shift) & 0xffu] + rank[r];
+      keys_out[dst] = key[r];
+      cls_out[dst] = cls[r];
+    }
+  }
+}
+
+// Sorted key i closes a run of equal keys.
+__device__ __forceinline__ bool roc_run_end(const unsigned int* __restrict__ keys, int64_t n, int64_t i) {
+  return i == n - 1 || keys[i + 1] != keys[i];
+}
+
+// sums[tile] = {run ends, genuine} in this tile of the sorted keys (kRocItems consecutive keys per thread).
+__global__ void __launch_bounds__(kRocThreads)
+roc_run_count_kernel(const unsigned int* __restrict__ keys, const unsigned char* __restrict__ cls, int64_t n,
+                     unsigned int* __restrict__ sums) {
+  const int64_t i0 = (int64_t)blockIdx.x * kRocTile + threadIdx.x * kRocItems;
+  unsigned int e = 0, g = 0;
+  for (int k = 0; k < kRocItems; ++k) {
+    const int64_t i = i0 + k;
+    if (i < n) {
+      e += roc_run_end(keys, n, i);
+      g += cls[i];
+    }
+  }
+  unsigned int te, tg;
+  roc_block_scan(e, &te);
+  roc_block_scan(g, &tg);
+  if (threadIdx.x == 0) {
+    sums[2 * (int64_t)blockIdx.x] = te;
+    sums[2 * (int64_t)blockIdx.x + 1] = tg;
+  }
+}
+
+// One block: exclusive scan, in place, of each of the `comps` interleaved columns of sums [n_tiles][comps]; column
+// totals -> totals[comps].
+__global__ void __launch_bounds__(kRocThreads)
+roc_tile_scan_kernel(unsigned int* __restrict__ sums, int64_t n_tiles, int comps, unsigned int* __restrict__ totals) {
+  for (int c = 0; c < comps; ++c) {
+    unsigned int carry = 0;
+    for (int64_t t0 = 0; t0 < n_tiles; t0 += kRocTile) {
+      const int64_t ti = t0 + threadIdx.x * kRocItems;
+      unsigned int s = 0;
+      for (int k = 0; k < kRocItems; ++k)
+        if (ti + k < n_tiles) s += sums[(ti + k) * comps + c];
+      unsigned int tot;
+      unsigned int run = carry + roc_block_scan(s, &tot);
+      for (int k = 0; k < kRocItems; ++k)
+        if (ti + k < n_tiles) {
+          const unsigned int v = sums[(ti + k) * comps + c];
+          sums[(ti + k) * comps + c] = run;
+          run += v;
+        }
+      carry += tot;
+    }
+    if (threadIdx.x == 0) totals[c] = carry;
+  }
+}
+
+// Run j of the sorted keys: tps[j] = genuine keys up to and including its last key, last[j] = that key's position.
+__global__ void __launch_bounds__(kRocThreads)
+roc_run_write_kernel(const unsigned int* __restrict__ keys, const unsigned char* __restrict__ cls, int64_t n,
+                     const unsigned int* __restrict__ sums, unsigned int* __restrict__ tps, unsigned int* __restrict__ last) {
+  const int64_t i0 = (int64_t)blockIdx.x * kRocTile + threadIdx.x * kRocItems;
+  unsigned int e = 0, g = 0;
+  for (int k = 0; k < kRocItems; ++k) {
+    const int64_t i = i0 + k;
+    if (i < n) {
+      e += roc_run_end(keys, n, i);
+      g += cls[i];
+    }
+  }
+  unsigned int t;
+  unsigned int j = sums[2 * (int64_t)blockIdx.x] + roc_block_scan(e, &t);
+  unsigned int gen = sums[2 * (int64_t)blockIdx.x + 1] + roc_block_scan(g, &t);
+  for (int k = 0; k < kRocItems; ++k) {
+    const int64_t i = i0 + k;
+    if (i < n) {
+      gen += cls[i];
+      if (roc_run_end(keys, n, i)) {
+        tps[j] = gen;
+        last[j] = (unsigned int)i;
+        ++j;
+      }
+    }
+  }
+}
+
+// sklearn's thinning (np.diff(fps, 2) or np.diff(tps, 2) nonzero): the first and the last of the m runs stay; an inner
+// run stays iff the next run has another genuine count or another size.
+__device__ __forceinline__ bool roc_keep(const unsigned int* __restrict__ tps, const unsigned int* __restrict__ last,
+                                         unsigned int m, int64_t j) {
+  if (j >= m) return false;
+  if (j == 0 || j == m - 1) return true;
+  return tps[j + 1] - tps[j] != tps[j] - tps[j - 1] || last[j + 1] - last[j] != last[j] - last[j - 1];
+}
+
+// sums[tile] = kept runs among this tile of kRocTile runs.
+__global__ void __launch_bounds__(kRocThreads)
+roc_keep_count_kernel(const unsigned int* __restrict__ tps, const unsigned int* __restrict__ last, const RocState* st,
+                      unsigned int* __restrict__ sums) {
+  const unsigned int m = st->run_totals[0];
+  const int64_t j0 = (int64_t)blockIdx.x * kRocTile + threadIdx.x * kRocItems;
+  unsigned int c = 0;
+  for (int k = 0; k < kRocItems; ++k) c += roc_keep(tps, last, m, j0 + k);
+  unsigned int t;
+  roc_block_scan(c, &t);
+  if (threadIdx.x == 0) sums[blockIdx.x] = t;
+}
+
+// The curve: point 0 is (0, 0) at +inf; kept run j becomes the next point, fpr = fps / n_imp, tpr = tps / n_gen.
+__global__ void __launch_bounds__(kRocThreads)
+roc_point_kernel(const unsigned int* __restrict__ keys, const unsigned int* __restrict__ tps,
+                 const unsigned int* __restrict__ last, const RocState* st, const unsigned int* __restrict__ sums,
+                 double* __restrict__ fpr, double* __restrict__ tpr, double* __restrict__ thresholds,
+                 int64_t* __restrict__ n_points, int64_t* __restrict__ counts) {
+  const unsigned int m = st->run_totals[0];
+  const int64_t j0 = (int64_t)blockIdx.x * kRocTile + threadIdx.x * kRocItems;
+  unsigned int c = 0;
+  for (int k = 0; k < kRocItems; ++k) c += roc_keep(tps, last, m, j0 + k);
+  unsigned int t;
+  unsigned int p = 1 + sums[blockIdx.x] + roc_block_scan(c, &t);
+  const double n_gen = (double)st->n_gen, n_imp = (double)st->n_imp;
+  for (int k = 0; k < kRocItems; ++k) {
+    const int64_t j = j0 + k;
+    if (roc_keep(tps, last, m, j)) {
+      const unsigned int tp = tps[j], fp = last[j] + 1 - tp;
+      fpr[p] = (double)fp / n_imp;
+      tpr[p] = (double)tp / n_gen;
+      thresholds[p] = roc_key_value(keys[last[j]]);
+      ++p;
+    }
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    fpr[0] = 0.0;
+    tpr[0] = 0.0;
+    thresholds[0] = (double)INFINITY;
+    *n_points = (int64_t)st->n_keep + 1;
+    counts[0] = (int64_t)st->n_gen;
+    counts[1] = (int64_t)st->n_imp;
+    counts[2] = (int64_t)st->n_bad;
+  }
+}
+
+// Workspace: the state, then 256-byte aligned arrays.
+struct RocLayout {
+  int64_t n_tiles, n_groups;
+  size_t keys[2], cls[2], hist, part, sums, tps, last, bytes;
+};
+
+static RocLayout roc_layout(int64_t n) {
+  RocLayout L;
+  L.n_tiles = (n + kRocTile - 1) / kRocTile;
+  L.n_groups = (L.n_tiles + kRocColTiles - 1) / kRocColTiles;
+  size_t o = 0;
+  auto take = [&o](size_t bytes) {
+    const size_t at = o;
+    o += (bytes + 255) & ~(size_t)255;
+    return at;
+  };
+  take(sizeof(RocState));
+  L.keys[0] = take(4 * (size_t)n);
+  L.keys[1] = take(4 * (size_t)n);
+  L.cls[0] = take((size_t)n);
+  L.cls[1] = take((size_t)n);
+  L.hist = take(4 * 256 * (size_t)L.n_tiles);
+  L.part = take(4 * 256 * (size_t)L.n_groups);
+  L.sums = take(4 * 2 * (size_t)L.n_tiles);
+  L.tps = take(4 * (size_t)n);
+  L.last = take(4 * (size_t)n);
+  L.bytes = o;
+  return L;
+}
+
 }  // namespace pfc
 
 using namespace pfc;
@@ -382,6 +744,67 @@ int pfc_tar_at_far(const float* scores, const unsigned char* issame, int64_t n, 
   tar_accept_kernel<<<(int)nb, kTarThreads, 0, st>>>(bits, issame, n, n_far, state);
   PFC_LAUNCH_CHECK();
   tar_finish_kernel<<<1, 32, 0, st>>>(state, n_far, counts, reinterpret_cast<unsigned int*>(thresholds));
+  PFC_LAUNCH_CHECK();
+  return 0;
+}
+
+size_t pfc_roc_curve_workspace_bytes(int64_t n) {
+  return roc_layout(n > 0 ? n : 0).bytes;
+}
+
+int pfc_roc_curve(const float* scores, const unsigned char* issame, int64_t n, double* fpr, double* tpr, double* thresholds,
+                  int64_t* n_points, int64_t* counts, void* workspace, size_t workspace_bytes, void* stream) {
+  if (int rc = require_sm100()) return rc;
+  NvtxScope nvtx_scope("pfc_roc_curve");
+  PFC_REQUIRE(scores && issame && fpr && tpr && thresholds && n_points && counts && workspace && n > 0, PFC_E_ARG,
+              "pfc_roc_curve: bad argument");
+  PFC_REQUIRE(reinterpret_cast<uintptr_t>(workspace) % 8 == 0, PFC_E_ARG, "pfc_roc_curve: workspace not 8-byte aligned");
+  PFC_REQUIRE(n < (1ll << 31), PFC_E_SHAPE, "pfc_roc_curve: more than 2^31 - 1 scores");
+  PFC_REQUIRE(workspace_bytes >= pfc_roc_curve_workspace_bytes(n), PFC_E_WORKSPACE, "pfc_roc_curve: workspace too small");
+  cudaStream_t st = as_stream(stream);
+  const RocLayout L = roc_layout(n);
+  char* ws = reinterpret_cast<char*>(workspace);
+  auto* state = reinterpret_cast<RocState*>(ws);
+  auto* hist = reinterpret_cast<unsigned int*>(ws + L.hist);
+  auto* part = reinterpret_cast<unsigned int*>(ws + L.part);
+  auto* sums = reinterpret_cast<unsigned int*>(ws + L.sums);
+  auto* tps = reinterpret_cast<unsigned int*>(ws + L.tps);
+  auto* last = reinterpret_cast<unsigned int*>(ws + L.last);
+  const auto* bits = reinterpret_cast<const unsigned int*>(scores);
+  const unsigned int nt = (unsigned int)L.n_tiles, ng = (unsigned int)L.n_groups;
+  PFC_CUDA(cudaMemsetAsync(state, 0, sizeof(RocState), st));
+  const unsigned int* keys = nullptr;
+  const unsigned char* cls = nullptr;
+  for (int pass = 0; pass < 4; ++pass) {       // LSD: digit 0 first; pass 0 reads the scores
+    const int shift = 8 * pass;
+    auto* keys_out = reinterpret_cast<unsigned int*>(ws + L.keys[pass & 1]);
+    auto* cls_out = reinterpret_cast<unsigned char*>(ws + L.cls[pass & 1]);
+    roc_hist_kernel<<<nt, kRocThreads, 0, st>>>(pass == 0 ? bits : nullptr, pass == 0 ? issame : nullptr, keys, n, shift,
+                                                hist, state);
+    PFC_LAUNCH_CHECK();
+    roc_col_sum_kernel<<<ng, kRocThreads, 0, st>>>(hist, L.n_tiles, part);
+    PFC_LAUNCH_CHECK();
+    roc_col_scan_kernel<<<1, kRocThreads, 0, st>>>(part, L.n_groups);
+    PFC_LAUNCH_CHECK();
+    roc_col_apply_kernel<<<ng, kRocThreads, 0, st>>>(hist, L.n_tiles, part);
+    PFC_LAUNCH_CHECK();
+    roc_scatter_kernel<<<nt, kRocThreads, 0, st>>>(pass == 0 ? bits : nullptr, pass == 0 ? issame : nullptr, keys, cls, n,
+                                                   shift, hist, keys_out, cls_out);
+    PFC_LAUNCH_CHECK();
+    keys = keys_out;
+    cls = cls_out;
+  }
+  roc_run_count_kernel<<<nt, kRocThreads, 0, st>>>(keys, cls, n, sums);
+  PFC_LAUNCH_CHECK();
+  roc_tile_scan_kernel<<<1, kRocThreads, 0, st>>>(sums, L.n_tiles, 2, state->run_totals);
+  PFC_LAUNCH_CHECK();
+  roc_run_write_kernel<<<nt, kRocThreads, 0, st>>>(keys, cls, n, sums, tps, last);
+  PFC_LAUNCH_CHECK();
+  roc_keep_count_kernel<<<nt, kRocThreads, 0, st>>>(tps, last, state, sums);
+  PFC_LAUNCH_CHECK();
+  roc_tile_scan_kernel<<<1, kRocThreads, 0, st>>>(sums, L.n_tiles, 1, &state->n_keep);
+  PFC_LAUNCH_CHECK();
+  roc_point_kernel<<<nt, kRocThreads, 0, st>>>(keys, tps, last, state, sums, fpr, tpr, thresholds, n_points, counts);
   PFC_LAUNCH_CHECK();
   return 0;
 }

@@ -4,6 +4,8 @@
     template_feats, template_ids = template_features(feats, templates, medias, weights)
     scores = pair_scores(template_feats, template_ids, p1, p2)
     for far_target, tar, far, threshold in tar_at_far(scores, issame): ...
+    fpr, tpr, thresholds = roc_curve(scores, issame)            # sklearn.metrics.roc_curve, element for element
+    for far_target, tar, far in tar_at_far_nearest(fpr, tpr): ...   # the insightface IJB scripts' TAR table
 
 The arithmetic is this repository's definition, pinned step by step (``include/fedfr_b200.h``, ``csrc/verify.cu``) so that
 a plain C restatement reproduces every feature and score bit for bit; it follows the usual insightface recipe (media
@@ -130,9 +132,9 @@ def tar_at_far(scores, issame, fars=DEFAULT_FARS):
     With n_imp impostor pairs and k = floor(f * n_imp), the threshold is the (k+1)-th largest impostor score (-inf when
     k >= n_imp) and a pair is accepted iff its score is above it, so ties at the threshold are rejected and the achieved
     far = accepted impostors / n_imp is at most f: the best operating point with FAR <= f.  -0.0 and +0.0 are one
-    value.  The sklearn-based IJB scripts instead read the nearest point of a thinned ROC curve; that lookup is not
-    reproduced.  scores fp32 [P], issame bool [P]; fars in (0, 1].  A NaN score, or no genuine or no impostor pair,
-    raises ValueError.  -> [(far_target, tar, far, threshold)]."""
+    value.  The sklearn-based IJB scripts instead read the nearest point of a thinned ROC curve: that read-out is
+    ``tar_at_far_nearest(*roc_curve(scores, issame)[:2])``.  scores fp32 [P], issame bool [P]; fars in (0, 1].  A NaN
+    score, or no genuine or no impostor pair, raises ValueError.  -> [(far_target, tar, far, threshold)]."""
     device = _device(scores)
     s = _on(scores, torch.float32, device).reshape(-1)
     y = (_on(issame, torch.int64, device).reshape(-1) != 0).to(torch.uint8)
@@ -155,3 +157,62 @@ def tar_at_far(scores, issame, fars=DEFAULT_FARS):
                                          N.ptr(thr), N.ptr(ws), ws.numel(), _stream(device)), "pfc_tar_at_far")
         result += tar_from_counts(counts.cpu().tolist(), thr.cpu().tolist(), chunk)
     return result
+
+
+def _numel(t):
+    return t.numel() if isinstance(t, torch.Tensor) else np.asarray(t).size
+
+
+def curve_length(counts, n_points):
+    """(counts [3] of pfc_roc_curve, n_points) -> n_points, or ValueError for NaN / inf scores or a missing class."""
+    n_gen, n_imp, n_nonfinite = (int(c) for c in counts)
+    if n_nonfinite:
+        raise ValueError("%d scores are NaN or infinite" % n_nonfinite)
+    if n_gen == 0 or n_imp == 0:
+        raise ValueError("roc_curve needs genuine and impostor pairs (got %d and %d)" % (n_gen, n_imp))
+    return int(n_points)
+
+
+def roc_curve(scores, issame):
+    """The ROC curve of the scores, equal element for element to ``sklearn.metrics.roc_curve(issame, scores)`` (with
+    its default ``drop_intermediate=True``), computed on the GPU by a radix sort of the scores and integer scans.
+
+    -0.0 and +0.0 are one value.  sklearn raises for NaN or infinite scores, and so does this.  Where sklearn only warns
+    and returns NaN rates (no genuine or no impostor pair), this raises ValueError.  The definition on counts is in
+    ``include/fedfr_b200.h``.  ``sklearn.metrics.auc(fpr, tpr)`` on the result gives the IJB scripts' AUC, and
+    ``tar_at_far_nearest(fpr, tpr)`` their TAR table.  scores fp32 [P], issame bool [P], CUDA tensors or numpy arrays.
+    -> (fpr, tpr, thresholds), float64 CUDA tensors of the curve's length; thresholds[0] = +inf."""
+    if _numel(scores) != _numel(issame):
+        raise ValueError("one issame flag per score")
+    if _numel(scores) == 0:
+        raise ValueError("roc_curve needs genuine and impostor pairs (got no scores)")
+    device = _device(scores)
+    s = _on(scores, torch.float32, device).reshape(-1)
+    y = (_on(issame, torch.int64, device).reshape(-1) != 0).to(torch.uint8)
+    n = s.numel()
+    ws = torch.empty(int(N.lib.pfc_roc_curve_workspace_bytes(n)), dtype=torch.uint8, device=device)
+    fpr, tpr, thr = (torch.empty(n + 1, dtype=torch.float64, device=device) for _ in range(3))
+    out = torch.empty(4, dtype=torch.int64, device=device)                  # counts [3], n_points
+    with torch.cuda.device(device):
+        N.check(N.lib.pfc_roc_curve(N.ptr(s), N.ptr(y), n, N.ptr(fpr), N.ptr(tpr), N.ptr(thr), N.ptr(out[3:]), N.ptr(out),
+                                    N.ptr(ws), ws.numel(), _stream(device)), "pfc_roc_curve")
+    host = out.cpu().tolist()
+    k = curve_length(host[:3], host[3])
+    return fpr[:k].clone(), tpr[:k].clone(), thr[:k].clone()
+
+
+def tar_at_far_nearest(fpr, tpr, fars=DEFAULT_FARS):
+    """TAR at each target FAR as the insightface IJB-B / IJB-C scripts print it (FedFR's ``ijbc_all.py`` and
+    ``ijbc_conti.py``): on the curve flipped end to end (largest tpr first at an equal fpr), the point whose fpr is
+    nearest to f, the first one on a tie.  Its FAR may lie above f; ``tar_at_far`` stays the exact FAR <= f operating
+    point.  fpr, tpr as ``roc_curve`` returns them (or sklearn's), tensors or numpy arrays; the lookup runs on the host.
+    -> [(far_target, tar, far_at_point)]."""
+    f = np.flipud(np.asarray(torch.as_tensor(fpr).cpu(), dtype=np.float64))
+    t = np.flipud(np.asarray(torch.as_tensor(tpr).cpu(), dtype=np.float64))
+    if f.size == 0 or f.shape != t.shape:
+        raise ValueError("fpr and tpr must be non-empty and of one length")
+    out = []
+    for far in fars:
+        i = int(np.argmin(np.abs(f - float(far))))
+        out.append((float(far), float(t[i]), float(f[i])))
+    return out

@@ -317,6 +317,24 @@ size_t pfc_tar_at_far_workspace_bytes(int64_t n);
 int pfc_tar_at_far(const float* scores, const unsigned char* issame, int64_t n, const double* fars_host, int n_far,
                    int64_t* counts, float* thresholds, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Exact ROC curve, element for element sklearn.metrics.roc_curve(issame, scores) (drop_intermediate=True).  scores fp32
+ * [n] (n < 2^31), issame uint8 [n] (nonzero = genuine).  Defined on counts, with no float sort order:
+ *   1. each score maps to the order-preserving uint32 key of pfc_tar_at_far, -0.0 folded onto +0.0;
+ *   2. walking the distinct keys in descending order, key j has g_j genuine and i_j impostor scores (exact counts);
+ *      tps = cumsum(g), fps = cumsum(i);
+ *   3. thinning keeps the first and the last key, and an inner key j iff g_{j+1} != g_j or i_{j+1} != i_j (sklearn's
+ *      nonzero second difference of fps / tps);
+ *   4. the point (0, 0) at threshold +inf comes first; then fpr = (double)fps / n_imp, tpr = (double)tps / n_gen (one
+ *      IEEE division each) and threshold = (double) of the key's fp32 value.
+ * Writes n_points[0] = the curve's length (<= n + 1) and fpr, tpr, thresholds [n_points] (room for n + 1 each; nothing
+ * past n_points is written), and counts int64 [3] = {n_gen, n_imp, n_nonfinite}: finite genuine, finite impostor, and
+ * NaN or +-inf scores.  The curve means nothing unless n_nonfinite == 0, n_gen > 0 and n_imp > 0 (fedfr_b200.verify
+ * raises otherwise).  Deterministic: integer counts and scans, no float atomics.  workspace:
+ * pfc_roc_curve_workspace_bytes(n) bytes (about 19 n), 8-byte aligned. */
+size_t pfc_roc_curve_workspace_bytes(int64_t n);
+int pfc_roc_curve(const float* scores, const unsigned char* issame, int64_t n, double* fpr, double* tpr, double* thresholds,
+                  int64_t* n_points, int64_t* counts, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

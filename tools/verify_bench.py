@@ -5,12 +5,13 @@
 Data: oracle.verify_oracle.ijbc_like, seeded synthetic arrays of the IJB-C 1:1 shape (227,630 images, 23,124 templates,
 15,658,489 pairs grouped by p1, 19,557 genuine), E = 512.  Each stage is timed with CUDA events over `reps` calls after
 a warm-up call: pooling (index plumbing included), pair scores (the pfc_pair_scores kernel alone, rows precomputed, and
-the public call with its id lookup), TAR@FAR at the six IJB-C FARs (public call, with the read-back of its counts).
+the public call with its id lookup), TAR@FAR at the six IJB-C FARs (public call, with the read-back of its counts), and
+the ROC curve (the pfc_roc_curve chain alone, buffers preallocated, and the public call with its read-back and copies).
 The 47 MB of template features stay in the 126 MB L2 between passes, as they would in use.  Counted work: bytes the
 pair kernel must read from L2 (every p2 row once per pair, every p1 row once per run of equal p1 in a 128-pair tile),
 and fp32->fp64 conversions (P * E).  Baseline: the float64 numpy restatement on the host cores in the same run (the
-pair scores on a seeded 1 M-pair sample, reported with its rate).  Prints the card name and power limit and writes
-OUT_DIR/verify_bench.json.
+pair scores on a seeded 1 M-pair sample, reported with its rate) and sklearn.metrics.roc_curve on all the scores.  The
+ROC curve must equal sklearn's array for array.  Prints the card name and power limit and writes OUT_DIR/verify_bench.json.
 """
 import argparse
 import json
@@ -21,6 +22,7 @@ import time
 
 import numpy as np
 import torch
+from sklearn.metrics import auc, roc_curve
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -101,6 +103,18 @@ def main():
     result = F.tar_at_far(scores, yd, fars)
     exact = result == O.tar_at_far(scores.cpu().numpy(), y, fars)
 
+    ws = torch.empty(int(N.lib.pfc_roc_curve_workspace_bytes(P)), dtype=torch.uint8, device=dev)
+    curve_bufs = [torch.empty(P + 1, dtype=torch.float64, device=dev) for _ in range(3)]
+    roc_out = torch.empty(4, dtype=torch.int64, device=dev)
+    y8 = yd.to(torch.uint8)
+
+    def roc_abi():
+        N.check(N.lib.pfc_roc_curve(N.ptr(scores), N.ptr(y8), P, *(N.ptr(b) for b in curve_bufs), N.ptr(roc_out[3:]),
+                                    N.ptr(roc_out), N.ptr(ws), ws.numel(), stream), "pfc_roc_curve")
+    ms_roc_abi = cuda_ms(roc_abi, args.reps)
+    ms_roc_call = cuda_ms(lambda: F.roc_curve(scores, yd), args.reps)
+    curve = [c.cpu().numpy() for c in F.roc_curve(scores, yd)]
+
     # counted work of the pair kernel
     r1h = r1.cpu().numpy()
     tile = np.arange(P) // 128
@@ -120,6 +134,10 @@ def main():
     t0 = time.perf_counter()
     O.tar_at_far(s_all, y, fars)
     s_np_tar = time.perf_counter() - t0
+    t0 = time.perf_counter()
+    sk = roc_curve(y, s_all)
+    s_sk_roc = time.perf_counter() - t0
+    roc_exact = all(np.array_equal(a, b) for a, b in zip(curve, sk))
     max_dev = float(np.abs(s_all[sample] - s64).max())
 
     rec = {
@@ -127,13 +145,18 @@ def main():
                                                       "genuine": int(y.sum()), "emb": int(E), "p1_runs_per_128_tiles": runs},
         "reps": args.reps,
         "ms": {"template_features": round(ms_pool, 4), "pair_scores_kernel": round(ms_pair_kernel, 4),
-               "pair_scores_call": round(ms_pair_call, 4), "tar_at_far_6_fars": round(ms_tar, 4)},
+               "pair_scores_call": round(ms_pair_call, 4), "tar_at_far_6_fars": round(ms_tar, 4),
+               "roc_curve_abi": round(ms_roc_abi, 4), "roc_curve_call": round(ms_roc_call, 4)},
         "pair_kernel": {"pairs_per_s": P / (ms_pair_kernel * 1e-3), "l2_bytes": l2_bytes,
                         "l2_bytes_per_s": l2_bytes / (ms_pair_kernel * 1e-3), "f2f_conversions": conversions,
                         "f2f_per_s": conversions / (ms_pair_kernel * 1e-3),
                         "f2f_per_clk_per_sm_at_max_clock": None},
         "tar_at_far": [{"far_target": f, "tar": tar, "far": far, "threshold": thr} for f, tar, far, thr in result],
         "tar_at_far_exact_vs_numpy": exact,
+        "roc_curve": {"points": int(curve[0].size), "exact_vs_sklearn": roc_exact, "auc": auc(curve[0], curve[1]),
+                      "sklearn_host_s": round(s_sk_roc, 3),
+                      "tar_at_far_nearest": [{"far_target": f, "tar": tar, "far": far}
+                                             for f, tar, far in F.tar_at_far_nearest(curve[0], curve[1], fars)]},
         "numpy_host": {"template_features_s": round(s_np_pool, 3), "pair_scores_sample": int(sample.size),
                        "pair_scores_sample_s": round(s_np_pairs_sample, 3),
                        "pair_scores_pairs_per_s": sample.size / s_np_pairs_sample, "tar_at_far_s": round(s_np_tar, 3),
@@ -149,6 +172,7 @@ def main():
         json.dump(rec, f, indent=1)
     print(json.dumps(rec))
     assert exact, "TAR@FAR differs from the numpy definition"
+    assert roc_exact, "the ROC curve differs from sklearn.metrics.roc_curve"
 
 
 if __name__ == "__main__":
