@@ -50,6 +50,7 @@ SIGNATURES = {
     "pfc_set_range_flag": (_i32, [_vp, _f32]),
     "pfc_bwd_prob_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "pfc_bwd_prob": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _f32, _f32, _i32, _f32, _vp, _vp, _i32, _vp, _sz, _vp, _sz, _vp]),
+    "pfc_spreadout_num_partials": (_i32, [_i64, _i32]),
     "pfc_spreadout_workspace_bytes": (_sz, [_i64, _i32]),
     "pfc_spreadout": (_i32, [_vp, _i64, _i32, _f32, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pfc_cosface_dense": (_i32, [_vp, _vp, _i64, _i64, _f32, _f32, _vp, _vp]),

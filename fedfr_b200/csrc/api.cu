@@ -22,6 +22,7 @@ int tc_bwd_prob(const void* x, const void* w_hat, const float* inv_norm, const i
                 size_t prob_ws_bytes, void* workspace, size_t workspace_bytes, cudaStream_t st);
 void tc_set_prob_split(int dx_sms, float dw_rate, int sweep_lead);
 size_t tc_spreadout_workspace_bytes(int64_t n, int emb);
+int tc_spreadout_num_partials(int64_t n);
 int tc_spreadout(const void* w_hat, int64_t n, int emb, float margin, float* part_max, float* part_sum, float* hw_out, void* workspace,
                  size_t workspace_bytes, cudaStream_t st);
 void tc_set_fwd_overlap(int chunks, int norm_blocks_per_sm);
@@ -134,6 +135,12 @@ int pfc_set_prob_split(int dx_sms, float dw_rate, int sweep_lead) {
 size_t pfc_spreadout_workspace_bytes(int64_t n, int emb) {
   if (n <= 0 || emb <= 0) return 0;
   return tc_spreadout_workspace_bytes(n, emb);
+}
+
+int pfc_spreadout_num_partials(int64_t n, int emb) {
+  (void)emb;
+  if (n <= 0) return 0;
+  return tc_spreadout_num_partials(n);
 }
 
 int pfc_spreadout(const void* w_hat, int64_t n, int emb, float margin, float* part_max, float* part_sum, float* hw_out, void* workspace,

@@ -2725,6 +2725,8 @@ size_t tc_spreadout_workspace_bytes(int64_t n, int emb) {
   const SpreadPlan pl = make_spread_plan(n, emb);
   return pl.scratch_bytes + pl.dxp_bytes;
 }
+// the hinge GEMM always runs on the CTA-pair kernel, whatever pfc_set_logits_pair / pfc_set_logits_tile select for the head
+int tc_spreadout_num_partials(int64_t n) { return 2 * pair_grid(n, n); }
 
 int tc_spreadout(const void* w_hat, int64_t n, int emb, float margin, float* part_max, float* part_sum, float* hw_out, void* workspace,
                  size_t workspace_bytes, cudaStream_t st) {

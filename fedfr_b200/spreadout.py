@@ -25,7 +25,7 @@ class _SpreadOutLoss(torch.autograd.Function):
         inv_norm = torch.empty(n, dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
             N.check(N.lib.pfc_normalize_rows(N.ptr(w), None, n, emb, N.ptr(w_hat), None, N.ptr(inv_norm), st), "pfc_normalize_rows")
-            n_part = N.lib.pfc_fwd_num_partials(n, n, emb, N.PATH_TENSOR)
+            n_part = N.lib.pfc_spreadout_num_partials(n, emb)
             part = torch.empty((2, n_part, n), dtype=torch.float32, device=dev)
             hw = torch.empty((n, emb), dtype=torch.float32, device=dev)
             nbytes = N.lib.pfc_spreadout_workspace_bytes(n, emb)

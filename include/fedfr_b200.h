@@ -193,11 +193,13 @@ int pfc_bwd_prob(const void* x, const void* w_hat, const float* inv_norm, const 
  * SpreadOut regulariser                                                 server.py:48-63 (SpreadOut_Module.forward)
  * ------------------------------------------------------------------------------------------------
  * similarity = w_hat . w_hat^T (w_hat = normalize(FC), bf16 [n, emb]); H_ij = relu(similarity_ij - margin) for i != j.
- *   part_sum [pfc_fwd_num_partials(n, n, emb, PFC_PATH_TENSOR), n]: partial sums of H_ij^2 per row (their total is the
- *            'sum' loss; part_max is scratch of the same shape);
+ *   part_sum [pfc_spreadout_num_partials(n, emb), n]: partial sums of H_ij^2 per row (their total is the 'sum' loss;
+ *            part_max is scratch of the same shape).  The count depends on the shape and the device alone, not on the
+ *            tuning knobs of the head's forward;
  *   hw_out   fp32 [n, emb] = H . w_hat.  d loss / d w_hat = 4 * hw_out (H is symmetric, each pair counted twice);
  *            the normalize backward to FC is row-wise and left to the caller.
  * The [n, n] similarity never exists; H lives as bf16 in `workspace` (pfc_spreadout_workspace_bytes, 1024-aligned). */
+int pfc_spreadout_num_partials(int64_t n, int emb);
 size_t pfc_spreadout_workspace_bytes(int64_t n, int emb);
 int pfc_spreadout(const void* w_hat, int64_t n, int emb, float margin, float* part_max, float* part_sum, float* hw_out,
                   void* workspace, size_t workspace_bytes, void* stream);
