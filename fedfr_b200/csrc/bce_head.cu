@@ -6,7 +6,7 @@
 //     logit = r * (g - m) + bias_c   when c is the row's class, else   r * (g + m) + bias_c            client.py:53-57
 //     gt    = (c == label_b), labels >= n_class (and -1) select no column                              client.py:48-52
 // backward from d logit (the caller's loss, losses.BCE_loss or anything else, runs in torch on the [B, C] logits):
-//     d cos = d logit * r * t * ((cos + 1) / 2)^(t - 1),    d bias_c = sum_b d logit
+//     d cos = d logit * r * t * ((cos + 1) / 2)^(t - 1),    d bias_c = sum_b d logit     ((cos + 1) / 2 clamped at 0)
 //     d f_b = ( sum_c d cos * w^_c  -  f^_b * sum_c d cos * cos ) / |f_b|       (matmul + normalize backward)
 //     d w_c = ( sum_b d cos * f^_b  -  w^_c * sum_b d cos * cos ) / |w_c|
 // The reference runs ~20 ATen kernels over [B, C] temporaries for this (two normalisations, a matmul, a [B, C+1] bool
@@ -69,7 +69,7 @@ bce_head_fwd_kernel(const float* __restrict__ feat, const float* __restrict__ we
       const float inf = 1.f / fmaxf(sqrtf(ff), kNormEps);
       const float inw = 1.f / fmaxf(sqrtf(ww), kNormEps);
       const float cs = fw * inf * inw;
-      const float u = (cs + 1.f) * 0.5f;
+      const float u = fmaxf((cs + 1.f) * 0.5f, 0.f);     // an antipodal pair can round below -1: powf would give NaN
       const float g = 2.f * pow_small(u, t) - 1.f;
       const bool pos = (bce_target_col(label[b], n_classes) == c);
       const float z = __fadd_rn(__fmul_rn(r, pos ? (g - m) : (g + m)), bias ? bias[c] : 0.f);
@@ -120,7 +120,7 @@ bce_head_bwd_kernel(const float* __restrict__ feat, const float* __restrict__ we
     for (int o = threadIdx.x; o < n_chunk; o += kBceThreads) {
       const int64_t e = row_role ? me * n_classes + (o0 + o) : (o0 + o) * n_classes + me;
       const float dz = dlogits[e], cs = cosine[e];
-      const float u = (cs + 1.f) * 0.5f;
+      const float u = fmaxf((cs + 1.f) * 0.5f, 0.f);
       const float dcos = dz * slope_scale * pow_small(u, t - 1.f);
       s_d[o] = dcos * inv_other[o0 + o];
       radial = fmaf(dcos, cs, radial);
@@ -142,6 +142,9 @@ bce_head_bwd_kernel(const float* __restrict__ feat, const float* __restrict__ we
     bias_sum = block_sum_128(bias_sum, scratch);
     if (threadIdx.x == 0) dbias[me] = bias_sum;
   }
+  // a row whose norm was clamped to eps (0 < |v| < 1e-12) has a constant denominator: autograd of F.normalize gives
+  // it no radial term (inv_me == 1 / eps marks it: the forward computed 1 / max(|v|, eps) with the same division)
+  if (inv_me >= 1.f / kNormEps) radial = 0.f;
   float* out = (row_role ? dfeat : dweight) + me * emb;
 #pragma unroll
   for (int j = 0; j < kBceMaxKpt; ++j) {

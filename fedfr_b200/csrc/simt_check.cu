@@ -142,16 +142,22 @@ __global__ void __launch_bounds__(256) gemm_kernel(const float* __restrict__ A, 
 }
 
 // dw_j = (dwh_j - w_hat_j (w_hat_j . dwh_j)) * inv_norm_j       one warp per row
+// A row whose norm was clamped to eps (0 < |w_j| < 1e-12) has w_hat_j = w_j / eps and a constant denominator: autograd of
+// F.normalize gives it dwh_j / eps with no radial term.  inv_norm_j == 1 / eps marks it (normalize_rows_warp computes
+// 1 / max(|w|, eps) with the same correctly rounded division); a norm within an ulp above eps may read as clamped too,
+// which is inside the rounding of the norm itself.
 __global__ void __launch_bounds__(256) normalize_bwd_kernel(const float* __restrict__ dwh, const float* __restrict__ w_hat,
                                                             const float* __restrict__ inv_norm, int64_t n_rows, int emb, float* __restrict__ dw,
                                                             int accumulate) {
   const int lane = threadIdx.x & 31;
   const int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (r >= n_rows) return;
-  float dot = 0.f;
-  for (int c = lane; c < emb; c += 32) dot += dwh[r * emb + c] * w_hat[r * emb + c];
-  dot = warp_sum(dot);
   const float inv = inv_norm[r];
+  float dot = 0.f;
+  if (inv < 1.f / 1e-12f) {
+    for (int c = lane; c < emb; c += 32) dot += dwh[r * emb + c] * w_hat[r * emb + c];
+    dot = warp_sum(dot);
+  }
   for (int c = lane; c < emb; c += 32) {
     float v = (dwh[r * emb + c] - w_hat[r * emb + c] * dot) * inv;
     if (accumulate) v += dw[r * emb + c];
@@ -179,10 +185,13 @@ int simt_fwd_stats(const float* x, const float* w_hat, const int64_t* label, int
   return 0;
 }
 
+// Class columns per backward chunk: a 64 MiB fp32 G scratch, at least one 64-column tile, and at most 65,535 tiles
+// (grad_logits_kernel puts the class tiles on gridDim.y).
 static int64_t check_chunk(int64_t n_rows, int64_t n_classes) {
   int64_t chunk = (64ll << 20) / (n_rows * 4);
   chunk = chunk / 64 * 64;
   if (chunk < 64) chunk = 64;
+  if (chunk > 65535ll * 64) chunk = 65535ll * 64;
   const int64_t cpad = (n_classes + 63) / 64 * 64;
   return chunk < cpad ? chunk : cpad;
 }

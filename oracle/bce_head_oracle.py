@@ -29,7 +29,7 @@ def forward(feat, weight, bias, labels, m, r, t):
     gt = torch.zeros_like(cosine, dtype=torch.bool)
     rows = torch.nonzero(col >= 0, as_tuple=True)[0]
     gt[rows, col[rows]] = True                                           # client.py:48-52
-    g = 2 * ((cosine + 1) / 2).pow(t) - 1                                # client.py:40
+    g = 2 * ((cosine + 1) / 2).clamp_min(0).pow(t) - 1                   # client.py:40 (an antipodal pair may round below -1)
     logits = torch.where(gt, r * (g - m), r * (g + m))                   # client.py:54,56
     if bias is not None:
         logits = logits + bias[None, :]                                  # client.py:57
@@ -38,11 +38,14 @@ def forward(feat, weight, bias, labels, m, r, t):
 
 def backward(feat, weight, cosine, nf, nw, dlogits, r, t):
     """d loss / d (feat, weight, bias) given d loss / d logits."""
-    dcos = dlogits * (r * t) * ((cosine + 1) / 2).pow(t - 1)
+    dcos = dlogits * (r * t) * ((cosine + 1) / 2).clamp_min(0).pow(t - 1)
     f_hat, w_hat = feat / nf[:, None], weight / nw[:, None]
     df_hat, dw_hat = dcos @ w_hat, dcos.t() @ f_hat
-    dfeat = (df_hat - f_hat * (f_hat * df_hat).sum(dim=1, keepdim=True)) / nf[:, None]
-    dweight = (dw_hat - w_hat * (w_hat * dw_hat).sum(dim=1, keepdim=True)) / nw[:, None]
+    # a norm clamped to EPS is a constant: autograd of F.normalize gives such a row no radial term
+    f_rad = torch.where(nf[:, None] > EPS, f_hat, torch.zeros_like(f_hat))
+    w_rad = torch.where(nw[:, None] > EPS, w_hat, torch.zeros_like(w_hat))
+    dfeat = (df_hat - f_rad * (f_hat * df_hat).sum(dim=1, keepdim=True)) / nf[:, None]
+    dweight = (dw_hat - w_rad * (w_hat * dw_hat).sum(dim=1, keepdim=True)) / nw[:, None]
     return dfeat, dweight, dlogits.sum(dim=0)
 
 
