@@ -57,6 +57,8 @@ SIGNATURES = {
     "pfc_arcface_dense": (_i32, [_vp, _vp, _i64, _i64, _f32, _f32, _vp]),
     "pfc_bce_head_fwd": (_i32, [_vp, _vp, _vp, _vp, _i64, _i64, _i32, _f32, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "pfc_bce_head_bwd": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _f32, _f32, _vp, _vp, _vp, _vp]),
+    "pfc_bce_loss_fwd": (_i32, [_vp, _vp, _vp, _vp, _i64, _i64, _i32, _f32, _f32, _f32, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "pfc_bce_loss_bwd": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _f32, _f32, _f32, _f32, _f32, _vp, _vp, _vp, _vp]),
     "pfc_similar_columns": (_i32, [_vp, _i64, _vp, _i64, _i32, _f32, _vp, _vp]),
     "pfc_roc_histogram": (_i32, [_vp, _vp, _i64, _vp, _vp, _i64, _i64, _i32, _vp, _vp]),
     "pfc_template_pool": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp]),

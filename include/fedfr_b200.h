@@ -264,6 +264,34 @@ int pfc_bce_head_bwd(const float* feat, const float* weight, const float* cosine
                      const float* inv_norm_w, const float* dlogits, int64_t n_rows, int64_t n_classes, int emb, float r,
                      float t, float* dfeat, float* dweight, float* dbias, void* stream);
 
+/* The head with losses.BCE_loss on top (losses.py:4-15, client.py:382,393), without the [n_rows, n_classes] logits.
+ * For row b and class c, cos, gt and the logit z are the fp32 values pfc_bce_head_fwd computes (same operations, same
+ * target-column rule, same clamp of (cos + 1) / 2 at 0).  With pos_coef = fl32(lam / r_loss) and
+ * neg_coef = fl32((1 - lam) / r_loss) (the Python doubles rounded once, as torch rounds a scalar factor; the reference
+ * uses lam = 0.7, r_loss = 30, which is not the head's r):
+ *   term(b, c) = gt ? pos_coef * log((1 + exp(-z)) + 1e-8) : neg_coef * log((1 + exp(z)) + 1e-8)
+ *   loss       = (sum over b in row order of row_loss[b]) / n_rows,   row_loss[b] = sum over c in class order of term(b, c)
+ * in fp32, each sum sequential from 0, so the loss is the same bits from run to run.  torch's literal formula, not log1p:
+ * an exp that overflows fp32 (|z| > ~88.7) gives an infinite loss, as in the reference.  n_rows == 0 gives a NaN loss
+ * (torch's mean of nothing); n_classes == 0 gives 0.
+ * Writes loss [1], row_loss [n_rows], and cosine, inv_norm_feat, inv_norm_w as pfc_bce_head_fwd does (inv_norm_feat even
+ * when n_classes == 0).  ticket: one device uint32 that is 0 before the call; the call returns it to 0.  Calls that may
+ * run at the same time need tickets of their own.  bias may be NULL.  emb <= 1024.  One launch. */
+int pfc_bce_loss_fwd(const float* feat, const float* weight, const float* bias, const int64_t* label, int64_t n_rows,
+                     int64_t n_classes, int emb, float m, float r, float t, float pos_coef, float neg_coef, float* loss,
+                     float* row_loss, unsigned int* ticket, float* cosine, float* inv_norm_feat, float* inv_norm_w,
+                     void* stream);
+/* Its autograd: pfc_bce_head_bwd with d loss / d z computed in the kernel from cosine, label and bias,
+ *   d z = ((grad_out[0] / n_rows) * coef) / ((1 + e) + 1e-8) * e,   e = exp(-z), coef = pos_coef, negated, on gt;
+ *                                                                   e = exp(z),  coef = neg_coef otherwise
+ * (autograd's order of operations; an overflowing exp gives NaN, as in the reference).  grad_out is a DEVICE scalar (the
+ * gradient arriving at the loss, e.g. 10 for 10 * loss), so no host synchronisation is needed.  Same outputs, NULL rules
+ * and size limits as pfc_bce_head_bwd; bias may be NULL.  One launch. */
+int pfc_bce_loss_bwd(const float* feat, const float* weight, const float* bias, const int64_t* label, const float* cosine,
+                     const float* inv_norm_feat, const float* inv_norm_w, const float* grad_out, int64_t n_rows,
+                     int64_t n_classes, int emb, float m, float r, float t, float pos_coef, float neg_coef, float* dfeat,
+                     float* dweight, float* dbias, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Hard-negative mining by similarity threshold              client.py:208-215 and client.py:232-235
  * ------------------------------------------------------------------------------------------------
