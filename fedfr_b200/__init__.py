@@ -9,8 +9,9 @@ from .losses import ArcFace, CosFace
 from .partial_fc import PartialFC
 from .roc import calc_ROC, roc_histogram, tpr_at_fpr
 from .spreadout import SpreadOut_Module
-from .verify import pair_scores, roc_curve, tar_at_far, tar_at_far_nearest, template_features
+from .verify import kfold_accuracy, pair_scores, roc_curve, tar_at_far, tar_at_far_nearest, template_features
 
 __all__ = ["PartialFC", "CosFace", "ArcFace", "FedPavg", "FedAvg_on_FC", "FedPavg_sharded", "FlatStateDict", "flatten_state_dict", "margin_cross_entropy", "MarginSoftmaxHead", "SpreadOut_Module",
            "BCE_module", "similar_columns", "hard_negative_ids", "calc_ROC", "roc_histogram", "tpr_at_fpr",
-           "template_features", "pair_scores", "tar_at_far", "roc_curve", "tar_at_far_nearest"]
+           "template_features", "pair_scores", "tar_at_far", "roc_curve", "tar_at_far_nearest",
+           "kfold_accuracy"]

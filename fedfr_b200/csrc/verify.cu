@@ -25,6 +25,14 @@
 // the sorted keys then cut it into runs of one key (tps = genuine up to the run's end, fps = its position + 1 - tps),
 // apply sklearn's thinning stencil to the runs and compact the kept points in order.  Integer counts and scans only: the
 // result does not depend on the schedule.
+//
+// K-fold verification accuracy (insightface's eval/verification.py evaluate / calculate_roc, the per-round LFW / CFP-FP
+// / AgeDB test): one warp per pair fuses, normalises and takes the squared distance of the two rows with the fp64 sums
+// pinned in the header, and bins the distance on the threshold grid by a binary search.  One CTA per fold then builds
+// the fold's integer histogram of bins by class (shared atomics) and adds it into the all-pairs totals (integer global
+// atomics); one CTA per fold scans its histogram and the totals into test and train counts, picks the first train
+// maximum and writes its accuracy and test rates; a last pass takes the fold-order mean of the rates.  Integer counts,
+// fixed-order sums: the result does not depend on the schedule.
 #include "common.cuh"
 #include "../../fedfr_b200/csrc/dot_chain.cuh"
 
@@ -674,6 +682,190 @@ static RocLayout roc_layout(int64_t n) {
   return L;
 }
 
+constexpr int kKfThreads = kRocThreads;        // the selection reuses roc_block_scan, which needs 256 threads
+constexpr int kKfPairsPerBlock = kKfThreads / 32;
+constexpr int kKfMaxEmb = 4096;
+constexpr int kKfMaxThr = 16384;
+constexpr int kKfWindow = 4096;                // histogram bins per class held in shared memory at once
+
+// Fused value x_k of row r: emb + flip (one fp32 add), or emb alone.
+__device__ __forceinline__ float kf_x(const float* __restrict__ emb, const float* __restrict__ flip, int64_t r, int E,
+                                      int k) {
+  const float e = emb[r * E + k];
+  return flip ? __fadd_rn(e, flip[r * E + k]) : e;
+}
+
+// The pinned warp sum of the lanes' fp64 partials: xor butterfly over 16, 8, 4, 2, 1.  a + b == b + a in IEEE
+// arithmetic, so every lane returns the same value.
+__device__ __forceinline__ double kf_warp_sum(double s) {
+  for (int o = 16; o > 0; o >>= 1) s = __dadd_rn(s, __shfl_xor_sync(0xffffffffu, s, o));
+  return s;
+}
+
+// Pair p = rows 2p and 2p+1: dist[p], and bins[p] = the first j with (double)dist < thr[j] (T if none, so a NaN
+// distance is never "same").  One warp per pair, grid-stride over the pairs.
+__global__ void __launch_bounds__(kKfThreads)
+kfold_dist_kernel(const float* __restrict__ emb, const float* __restrict__ flip, int64_t n_pairs, int E,
+                  const double* __restrict__ thr, int T, float* __restrict__ dist, int* __restrict__ bins) {
+  const int lane = threadIdx.x & 31;
+  for (int64_t p = (int64_t)blockIdx.x * kKfPairsPerBlock + (threadIdx.x >> 5); p < n_pairs;
+       p += (int64_t)gridDim.x * kKfPairsPerBlock) {
+    const int64_t r1 = 2 * p, r2 = 2 * p + 1;
+    double s1 = 0.0, s2 = 0.0;
+    for (int k = lane; k < E; k += 32) {
+      const double a = (double)kf_x(emb, flip, r1, E, k), b = (double)kf_x(emb, flip, r2, E, k);
+      s1 = __dadd_rn(s1, __dmul_rn(a, a));
+      s2 = __dadd_rn(s2, __dmul_rn(b, b));
+    }
+    float n1 = (float)sqrt(kf_warp_sum(s1)), n2 = (float)sqrt(kf_warp_sum(s2));
+    if (n1 == 0.f) n1 = 1.f;
+    if (n2 == 0.f) n2 = 1.f;
+    double s = 0.0;
+    for (int k = lane; k < E; k += 32) {
+      const float d = kf_x(emb, flip, r1, E, k) / n1 - kf_x(emb, flip, r2, E, k) / n2;
+      s = __dadd_rn(s, __dmul_rn((double)d, (double)d));
+    }
+    s = kf_warp_sum(s);
+    if (lane == 0) {
+      const float d = (float)s;
+      int lo = 0, hi = T;
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if ((double)d < thr[mid]) hi = mid;
+        else lo = mid + 1;
+      }
+      dist[p] = d;
+      bins[p] = lo;
+    }
+  }
+}
+
+// sklearn's KFold(F, shuffle=False): fold f tests pairs [lo, hi); the first P % F folds hold one pair more.
+__device__ __forceinline__ void kf_fold_range(int64_t n_pairs, int64_t F, int64_t f, int64_t* lo, int64_t* hi) {
+  const int64_t q = n_pairs / F, r = n_pairs % F;
+  *lo = f * q + (f < r ? f : r);
+  *hi = *lo + q + (f < r ? 1 : 0);
+}
+
+// One CTA per fold: hist[f][c][b] = test pairs of class c (0 genuine, 1 impostor) with bin b, b = 0 ... T; the same
+// counts are added into totals[c][b].  Bins are counted kKfWindow at a time in shared memory.
+__global__ void __launch_bounds__(kKfThreads)
+kfold_hist_kernel(const int* __restrict__ bins, const unsigned char* __restrict__ issame, int64_t n_pairs, int64_t F,
+                  int T, int* __restrict__ hist, int* __restrict__ totals) {
+  __shared__ int sh[2][kKfWindow];
+  const int64_t f = blockIdx.x;
+  int64_t lo, hi;
+  kf_fold_range(n_pairs, F, f, &lo, &hi);
+  int* h = hist + f * 2 * (T + 1);
+  for (int w0 = 0; w0 <= T; w0 += kKfWindow) {
+    const int nw = T + 1 - w0 < kKfWindow ? T + 1 - w0 : kKfWindow;
+    for (int i = threadIdx.x; i < 2 * kKfWindow; i += kKfThreads) sh[i / kKfWindow][i % kKfWindow] = 0;
+    __syncthreads();
+    for (int64_t p = lo + threadIdx.x; p < hi; p += kKfThreads) {
+      const int b = bins[p] - w0;
+      if (b >= 0 && b < nw) atomicAdd(&sh[issame[p] ? 0 : 1][b], 1);
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nw; i += kKfThreads)
+      for (int c = 0; c < 2; ++c) {
+        const int v = sh[c][i];
+        h[c * (T + 1) + w0 + i] = v;
+        if (v) atomicAdd(&totals[c * (T + 1) + w0 + i], v);
+      }
+    __syncthreads();                           // sh is cleared for the next window
+  }
+}
+
+// Counts of one class at one threshold, as insightface's calculate_accuracy takes them.
+__device__ __forceinline__ double kf_rate(unsigned int hit, unsigned int n) {
+  return n ? (double)hit / (double)n : 0.0;
+}
+
+// One CTA per fold.  Thread t walks thresholds [t C, (t + 1) C) in order with the inclusive counts of bins <= j: test
+// genuine / impostor from hist[f], all-pairs from totals; train = all - test (train = test when F = 1).  It writes the
+// test rates rates[f][0 tpr, 1 fpr][j] and keeps its first maximum of the train tp + tn; thread 0 then takes the first
+// maximum over the threads in order, which is the first over j.
+__global__ void __launch_bounds__(kKfThreads)
+kfold_select_kernel(const int* __restrict__ hist, const int* __restrict__ totals, int64_t F, int T,
+                    const double* __restrict__ thr, double* __restrict__ rates, double* __restrict__ accuracy,
+                    double* __restrict__ best_thr) {
+  __shared__ unsigned int best_val[kKfThreads], best_j[kKfThreads], best_test[kKfThreads];
+  const int64_t f = blockIdx.x;
+  const int* hg = hist + f * 2 * (T + 1);
+  const int* hi = hg + (T + 1);
+  const int* tg = totals;
+  const int* ti = totals + (T + 1);
+  const int C = (T + kKfThreads - 1) / kKfThreads;
+  const int j0 = threadIdx.x * C < T ? threadIdx.x * C : T;
+  const int j1 = j0 + C < T ? j0 + C : T;
+  unsigned int s[4] = {0u, 0u, 0u, 0u};
+  for (int j = j0; j < j1; ++j) {
+    s[0] += hg[j]; s[1] += hi[j]; s[2] += tg[j]; s[3] += ti[j];
+  }
+  unsigned int cum[4], all[4];
+  for (int q = 0; q < 4; ++q) cum[q] = roc_block_scan(s[q], &all[q]);
+  // class sizes: bins 0 ... T - 1 plus bin T (never "same")
+  const unsigned int n_gen_te = all[0] + hg[T], n_imp_te = all[1] + hi[T], n_imp = all[3] + ti[T];
+  const bool one_fold = F == 1;
+  double* r_tpr = rates + f * 2 * (int64_t)T;
+  double* r_fpr = r_tpr + T;
+  unsigned int bv = 0u, bj = 0xffffffffu, bt = 0u;
+  for (int j = j0; j < j1; ++j) {
+    cum[0] += hg[j]; cum[1] += hi[j]; cum[2] += tg[j]; cum[3] += ti[j];
+    const unsigned int tp = cum[0], fp = cum[1];                      // test: predicted same iff bin <= j
+    const unsigned int tn = n_imp_te - fp;
+    const unsigned int train = one_fold ? tp + tn : (cum[2] - tp) + ((n_imp - n_imp_te) - (cum[3] - fp));
+    if (bj == 0xffffffffu || train > bv) { bv = train; bj = (unsigned int)j; bt = tp + tn; }
+    r_tpr[j] = kf_rate(tp, n_gen_te);
+    r_fpr[j] = kf_rate(fp, n_imp_te);
+  }
+  best_val[threadIdx.x] = bv;
+  best_j[threadIdx.x] = bj;
+  best_test[threadIdx.x] = bt;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int w = -1;
+    for (int t = 0; t < kKfThreads; ++t)
+      if (best_j[t] != 0xffffffffu && (w < 0 || best_val[t] > best_val[w])) w = t;
+    accuracy[f] = (double)best_test[w] / (double)(n_gen_te + n_imp_te);
+    best_thr[f] = thr[best_j[w]];
+  }
+}
+
+// tpr[j] = (rates[0][0][j] + rates[1][0][j] + ...) / F in fold order (np.mean(tprs, 0)); fpr the same.
+__global__ void __launch_bounds__(kKfThreads)
+kfold_mean_kernel(const double* __restrict__ rates, int64_t F, int T, double* __restrict__ tpr, double* __restrict__ fpr) {
+  const int j = blockIdx.x * kKfThreads + threadIdx.x;
+  if (j >= T) return;
+  double st = 0.0, sf = 0.0;
+  for (int64_t f = 0; f < F; ++f) {
+    st = __dadd_rn(st, rates[f * 2 * T + j]);
+    sf = __dadd_rn(sf, rates[f * 2 * T + T + j]);
+  }
+  tpr[j] = st / (double)F;
+  fpr[j] = sf / (double)F;
+}
+
+struct KfoldLayout {
+  size_t bins, hist, totals, rates, bytes;
+};
+
+static KfoldLayout kfold_layout(int64_t n_pairs, int T, int64_t F) {
+  KfoldLayout L;
+  size_t o = 0;
+  auto take = [&o](size_t bytes) {
+    const size_t at = o;
+    o += (bytes + 255) & ~(size_t)255;
+    return at;
+  };
+  L.bins = take(4 * (size_t)n_pairs);
+  L.hist = take(4 * 2 * (size_t)F * (size_t)(T + 1));
+  L.totals = take(4 * 2 * (size_t)(T + 1));
+  L.rates = take(8 * 2 * (size_t)F * (size_t)T);
+  L.bytes = o;
+  return L;
+}
+
 }  // namespace pfc
 
 using namespace pfc;
@@ -805,6 +997,47 @@ int pfc_roc_curve(const float* scores, const unsigned char* issame, int64_t n, d
   roc_tile_scan_kernel<<<1, kRocThreads, 0, st>>>(sums, L.n_tiles, 1, &state->n_keep);
   PFC_LAUNCH_CHECK();
   roc_point_kernel<<<nt, kRocThreads, 0, st>>>(keys, tps, last, state, sums, fpr, tpr, thresholds, n_points, counts);
+  PFC_LAUNCH_CHECK();
+  return 0;
+}
+
+size_t pfc_kfold_workspace_bytes(int64_t n_pairs, int n_thresholds, int64_t nfolds) {
+  return kfold_layout(n_pairs > 0 ? n_pairs : 0, n_thresholds > 0 ? n_thresholds : 0, nfolds > 0 ? nfolds : 0).bytes;
+}
+
+int pfc_kfold_accuracy(const float* emb, const float* flip, const unsigned char* issame, int64_t n_pairs, int emb_dim,
+                       const double* thr, int n_thresholds, int64_t nfolds, float* dist, double* accuracy, double* best_thr,
+                       double* tpr, double* fpr, void* workspace, size_t workspace_bytes, void* stream) {
+  if (int rc = require_sm100()) return rc;
+  NvtxScope nvtx_scope("pfc_kfold_accuracy");
+  PFC_REQUIRE(emb && issame && thr && dist && accuracy && best_thr && tpr && fpr && workspace, PFC_E_ARG,
+              "pfc_kfold_accuracy: null pointer");
+  PFC_REQUIRE(n_pairs > 0 && emb_dim > 0 && n_thresholds > 0 && nfolds >= 1 && nfolds <= n_pairs, PFC_E_ARG,
+              "pfc_kfold_accuracy: bad size (need P >= 1, emb >= 1, T >= 1, 1 <= nfolds <= P)");
+  PFC_REQUIRE(reinterpret_cast<uintptr_t>(workspace) % 8 == 0, PFC_E_ARG, "pfc_kfold_accuracy: workspace not 8-byte aligned");
+  PFC_REQUIRE(emb_dim <= kKfMaxEmb && n_pairs < (1ll << 31) && n_thresholds <= kKfMaxThr, PFC_E_SHAPE,
+              "pfc_kfold_accuracy: emb > 4096, P >= 2^31 or more than 16384 thresholds");
+  PFC_REQUIRE(workspace_bytes >= pfc_kfold_workspace_bytes(n_pairs, n_thresholds, nfolds), PFC_E_WORKSPACE,
+              "pfc_kfold_accuracy: workspace too small");
+  cudaStream_t st = as_stream(stream);
+  const KfoldLayout L = kfold_layout(n_pairs, n_thresholds, nfolds);
+  char* ws = reinterpret_cast<char*>(workspace);
+  auto* bins = reinterpret_cast<int*>(ws + L.bins);
+  auto* hist = reinterpret_cast<int*>(ws + L.hist);
+  auto* totals = reinterpret_cast<int*>(ws + L.totals);
+  auto* rates = reinterpret_cast<double*>(ws + L.rates);
+  PFC_CUDA(cudaMemsetAsync(totals, 0, 4 * 2 * (size_t)(n_thresholds + 1), st));
+  int64_t nb = (n_pairs + kKfPairsPerBlock - 1) / kKfPairsPerBlock;
+  if (nb > 16 * sm_count()) nb = 16 * sm_count();
+  kfold_dist_kernel<<<(unsigned int)nb, kKfThreads, 0, st>>>(emb, flip, n_pairs, emb_dim, thr, n_thresholds, dist, bins);
+  PFC_LAUNCH_CHECK();
+  kfold_hist_kernel<<<(unsigned int)nfolds, kKfThreads, 0, st>>>(bins, issame, n_pairs, nfolds, n_thresholds, hist, totals);
+  PFC_LAUNCH_CHECK();
+  kfold_select_kernel<<<(unsigned int)nfolds, kKfThreads, 0, st>>>(hist, totals, nfolds, n_thresholds, thr, rates,
+                                                                   accuracy, best_thr);
+  PFC_LAUNCH_CHECK();
+  kfold_mean_kernel<<<(unsigned int)((n_thresholds + kKfThreads - 1) / kKfThreads), kKfThreads, 0, st>>>(
+      rates, nfolds, n_thresholds, tpr, fpr);
   PFC_LAUNCH_CHECK();
   return 0;
 }

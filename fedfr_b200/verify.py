@@ -6,6 +6,7 @@
     for far_target, tar, far, threshold in tar_at_far(scores, issame): ...
     fpr, tpr, thresholds = roc_curve(scores, issame)            # sklearn.metrics.roc_curve, element for element
     for far_target, tar, far in tar_at_far_nearest(fpr, tpr): ...   # the insightface IJB scripts' TAR table
+    acc, best_thr, tpr, fpr = kfold_accuracy(emb, issame, flipped)  # the per-round LFW / CFP-FP / AgeDB K-fold test
 
 The arithmetic is this repository's definition, pinned step by step (``include/fedfr_b200.h``, ``csrc/verify.cu``) so that
 a plain C restatement reproduces every feature and score bit for bit; it follows the usual insightface recipe (media
@@ -216,3 +217,65 @@ def tar_at_far_nearest(fpr, tpr, fars=DEFAULT_FARS):
         i = int(np.argmin(np.abs(f - float(far))))
         out.append((float(far), float(t[i]), float(f[i])))
     return out
+
+
+def kfold_thresholds(thresholds=None):
+    """The threshold grid as a validated float64 numpy array: ``np.arange(0, 4, 0.01)`` (insightface's ``evaluate``)
+    when None.  ValueError unless it is 1-D, non-empty, finite and strictly ascending.  A CUDA tensor is copied to the
+    host to be checked, which waits for the device."""
+    if thresholds is None:
+        return np.arange(0, 4, 0.01)
+    if isinstance(thresholds, torch.Tensor):
+        thresholds = thresholds.detach().cpu().numpy()
+    t = np.asarray(thresholds, dtype=np.float64)
+    if t.ndim != 1 or t.size == 0:
+        raise ValueError("thresholds must be a non-empty 1-D array")
+    if not np.isfinite(t).all():
+        raise ValueError("thresholds must be finite")
+    if not (t[1:] > t[:-1]).all():
+        raise ValueError("thresholds must be strictly ascending")
+    return np.ascontiguousarray(t)
+
+
+def kfold_accuracy(embeddings, issame, flipped=None, nfolds=10, thresholds=None):
+    """The K-fold verification accuracy of the per-round LFW / CFP-FP / AgeDB test (insightface's
+    ``eval/verification.py``: ``test()``'s flip fusion and normalisation, then ``evaluate`` / ``calculate_roc``), exact
+    on integer counts.
+
+    embeddings fp32 [2P, E] (rows 2p and 2p+1 are pair p); flipped fp32 [2P, E] (the embeddings of the flipped images,
+    added to ``embeddings`` before normalising) or None; issame bool [P]; folds are sklearn's ``KFold(nfolds)`` without
+    shuffling (nfolds = 1: train = test = all pairs); thresholds float64 [T], strictly ascending, default
+    ``np.arange(0, 4, 0.01)``.  CUDA tensors or numpy arrays.  A pair is predicted "same" at threshold t iff its squared
+    distance is < t.  The definition, with its pinned fp64 sums, is in ``include/fedfr_b200.h``: on the same distances,
+    every output equals the numpy recipe's element for element.  Nothing is copied back to the host, so the call does not
+    wait for the device (unless ``thresholds`` is a CUDA tensor, which is checked on the host).
+
+    -> (accuracy [nfolds], best_thresholds [nfolds], tpr [T], fpr [T]), float64 CUDA tensors.  ``test()``'s
+    ``acc2, std2`` are ``accuracy.mean(), accuracy.std(correction=0)`` (np.std's ddof=0; torch's default is 1)."""
+    shape = tuple(embeddings.shape) if isinstance(embeddings, torch.Tensor) else np.shape(embeddings)
+    if len(shape) != 2 or shape[0] % 2 or shape[1] == 0:
+        raise ValueError("embeddings must be [2P, E]: an even number of rows, pair p in rows 2p and 2p+1")
+    if flipped is not None and (tuple(flipped.shape) if isinstance(flipped, torch.Tensor) else np.shape(flipped)) != shape:
+        raise ValueError("flipped must have the shape of embeddings")
+    n_pairs = shape[0] // 2
+    if _numel(issame) != n_pairs:
+        raise ValueError("one issame flag per pair (%d pairs, got %d flags)" % (n_pairs, _numel(issame)))
+    nfolds = int(nfolds)
+    if not 1 <= nfolds <= n_pairs:
+        raise ValueError("nfolds must lie in [1, %d] (the number of pairs), got %d" % (n_pairs, nfolds))
+    thr_host = kfold_thresholds(thresholds)
+    device = _device(embeddings)
+    e = _on(embeddings, torch.float32, device)
+    fl = None if flipped is None else _on(flipped, torch.float32, device)
+    y = (_on(issame, torch.int64, device).reshape(-1) != 0).to(torch.uint8)
+    thr = torch.from_numpy(thr_host).pin_memory().to(device, non_blocking=True)
+    n_thr = thr.numel()
+    ws = torch.empty(int(N.lib.pfc_kfold_workspace_bytes(n_pairs, n_thr, nfolds)), dtype=torch.uint8, device=device)
+    dist = torch.empty(n_pairs, dtype=torch.float32, device=device)
+    acc, best = (torch.empty(nfolds, dtype=torch.float64, device=device) for _ in range(2))
+    tpr, fpr = (torch.empty(n_thr, dtype=torch.float64, device=device) for _ in range(2))
+    with torch.cuda.device(device):
+        N.check(N.lib.pfc_kfold_accuracy(N.ptr(e), N.ptr(fl), N.ptr(y), n_pairs, e.shape[1], N.ptr(thr), n_thr, nfolds,
+                                         N.ptr(dist), N.ptr(acc), N.ptr(best), N.ptr(tpr), N.ptr(fpr), N.ptr(ws),
+                                         ws.numel(), _stream(device)), "pfc_kfold_accuracy")
+    return acc, best, tpr, fpr

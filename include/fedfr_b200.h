@@ -365,6 +365,39 @@ size_t pfc_roc_curve_workspace_bytes(int64_t n);
 int pfc_roc_curve(const float* scores, const unsigned char* issame, int64_t n, double* fpr, double* tpr, double* thresholds,
                   int64_t* n_points, int64_t* counts, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * K-fold verification accuracy (LFW / CFP-FP / AgeDB)      eval/verification.py test() / evaluate() / calculate_roc
+ * ------------------------------------------------------------------------------------------------
+ * The per-round small-set test, exact on integer counts.  emb fp32 [2P, emb] (rows 2p and 2p+1 are pair p: evaluate's
+ * embeddings[0::2] / [1::2]), flip fp32 [2P, emb] or NULL, issame uint8 [P] (nonzero = genuine), thr fp64 [T] strictly
+ * ascending (the caller's grid, e.g. np.arange(0, 4, 0.01); never recomputed here), F = nfolds.
+ *   1. fused row: x_k = fl32(emb_k + flip_k), or emb_k when flip is NULL;
+ *   2. sklearn.preprocessing.normalize's formula with a pinned fp64 sum of squares:
+ *        nrm = (float)sqrt(sum_k (double)x_k^2), nrm = 1 when it is 0, xh_k = x_k / nrm (one fp32 IEEE division).
+ *      The sum: lane l of 32 adds k = l, l + 32, l + 64, ... in ascending order (fp64, round to nearest), then the 32
+ *      partials are added by an xor butterfly s_l = s_l + s_{l^o} for o = 16, 8, 4, 2, 1 (all lanes end equal);
+ *   3. dist[p] = (float)(sum_k (double)fl32(xh1_k - xh2_k)^2), summed in the same order (the fp64 square of an fp32
+ *      difference is exact);
+ *   4. b_p = #{j : !((double)dist[p] < thr_j)}: pair p is predicted "same" at threshold j iff dist < thr_j iff j >= b_p
+ *      (numpy 2's np.less(dist, thr_j) with an np.float64 threshold; a NaN distance gets b_p = T, never "same");
+ *   5. folds are sklearn's KFold(F, shuffle=False): contiguous test blocks of P / F pairs, the first P % F one longer;
+ *      train is the complement.  F = 1 is insightface's LFold: train = test = all pairs;
+ *   6. per fold f and threshold j, integer tp / fp / tn / fn on train and on test.  best_f = the first j maximising the
+ *      train tp + tn (np.argmax of the train accuracy); accuracy[f] = (double)(tp + tn)_test[best_f] / n_test;
+ *      best_thr[f] = thr[best_f]; the test rates tpr_fj = (double)tp / (tp + fn) and fpr_fj = (double)fp / (fp + tn),
+ *      0 when the denominator is 0;
+ *   7. tpr[j] = (tpr_0j + tpr_1j + ... + tpr_(F-1)j) / F, added in fold order, then one division (np.mean(tprs, 0));
+ *      fpr the same.
+ * Writes dist fp32 [P], accuracy and best_thr fp64 [F], tpr and fpr fp64 [T].  Limits: 1 <= emb <= 4096, 1 <= P < 2^31,
+ * 1 <= T <= 16384, 1 <= F <= P.  Deterministic: integer histograms (shared-memory atomics), fixed-order scans and sums,
+ * no sort, no float atomics; the host is never synchronised.  workspace: pfc_kfold_workspace_bytes(P, T, F) bytes
+ * (about 4 P + 24 F T: the bins, the per-fold histograms and the per-fold rates), 8-byte aligned.  VAL@FAR
+ * (calculate_val) and the pca > 0 branch are not part of this call. */
+size_t pfc_kfold_workspace_bytes(int64_t n_pairs, int n_thresholds, int64_t nfolds);
+int pfc_kfold_accuracy(const float* emb, const float* flip, const unsigned char* issame, int64_t n_pairs, int emb_dim,
+                       const double* thr, int n_thresholds, int64_t nfolds, float* dist, double* accuracy, double* best_thr,
+                       double* tpr, double* fpr, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
