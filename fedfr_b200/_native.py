@@ -69,6 +69,8 @@ SIGNATURES = {
     "pfc_roc_curve": (_i32, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pfc_kfold_workspace_bytes": (_sz, [_i64, _i32, _i64]),
     "pfc_kfold_accuracy": (_i32, [_vp, _vp, _vp, _i64, _i32, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "pfc_identify_workspace_bytes": (_sz, [_i64]),
+    "pfc_identify": (_i32, [_vp, _i64, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "fedavg_table_bytes": (_sz, [_i32, _i32]),
     "fedavg_weighted_sum": (_i32, [_vp, _vp, _vp, _vp, _i32, _vp, _i32, _vp, _sz, _vp]),
     "fedavg_blend": (_i32, [_vp, _vp, _f32, _f32, _i64, _vp, _vp]),

@@ -17,9 +17,9 @@
 namespace pfc {
 
 constexpr int kRocBins = 2001;
-constexpr int kRocTile = 64;
-constexpr int kRocK = 32;
-constexpr int kRocThreads = 256;
+constexpr int kRocTile = kChainTile;      // the exact kernel's tile loop is tile_chain (dot_chain.cuh)
+constexpr int kRocK = kChainK;
+constexpr int kRocThreads = kChainThreads;
 constexpr int kRocFlushTiles = 1 << 19;   // 2^19 tiles * 4096 pairs < 2^32: the shared counters cannot wrap
 
 __device__ __forceinline__ void roc_flush(unsigned int* h, unsigned long long* hist) {
@@ -55,39 +55,7 @@ roc_hist_kernel(const float* __restrict__ feature, const int32_t* __restrict__ l
     if (j_last <= sub_offset + i0) continue;          // no pair with i < j in this tile (uniform over the CTA)
 
     double acc[4][4];
-#pragma unroll
-    for (int u = 0; u < 4; ++u)
-#pragma unroll
-      for (int v = 0; v < 4; ++v) acc[u][v] = 0.0;
-
-    for (int k0 = 0; k0 < emb; k0 += kRocK) {
-      __syncthreads();                                // the previous slice (or tile) has been consumed
-      {
-        const int kk = tid & 31;
-        const bool k_ok = (k0 + kk) < emb;
-#pragma unroll
-        for (int r = 0; r < kRocTile / 8; ++r) {
-          const int row = (tid >> 5) + 8 * r;
-          const int64_t gi = i0 + row, gj = j0 + row;
-          As[row][kk] = (k_ok && gi < n_sub) ? sub[gi * emb + k0 + kk] : 0.f;
-          Bs[row][kk] = (k_ok && gj < n) ? feature[gj * emb + k0 + kk] : 0.f;
-        }
-      }
-      __syncthreads();
-      const int kc = (emb - k0 < kRocK) ? emb - k0 : kRocK;
-#pragma unroll 4
-      for (int kk = 0; kk < kc; ++kk) {
-        float a[4], b[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) a[u] = As[ty + 16 * u][kk];
-#pragma unroll
-        for (int v = 0; v < 4; ++v) b[v] = Bs[tx + 16 * v][kk];
-#pragma unroll
-        for (int u = 0; u < 4; ++u)
-#pragma unroll
-          for (int v = 0; v < 4; ++v) acc[u][v] = __dadd_rn(acc[u][v], (double)__fmul_rn(a[u], b[v]));
-      }
-    }
+    tile_chain(sub, n_sub, i0, feature, n, j0, emb, As, Bs, acc);
 
 #pragma unroll
     for (int u = 0; u < 4; ++u) {

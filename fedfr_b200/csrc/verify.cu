@@ -13,11 +13,11 @@
 // per thread) and stages 32-wide k slices of their rows in shared memory; the distinct runs of row1 in the tile are
 // staged once each, so a pair list grouped by its first template (as IJB-C's is) reads that row once per tile.
 //
-// TAR@FAR: scores map to order-preserving uint32 keys (-0.0 folded onto +0.0, NaN counted and left out).  A 4 x 8-bit
-// radix select over the impostor keys finds the (k+1)-th largest for up to 8 FARs at once: per pass, the unresolved
-// selections with the same key prefix share one histogram (prefixes of one length are equal or disjoint, so each key
-// lands in at most one), counted with warp-aggregated shared atomics; the last block to finish a pass picks the bins.
-// One counting pass then accepts score > threshold for every FAR.  No sort of the scores.
+// TAR@FAR: scores map to order-preserving uint32 keys (tar_key in score_key.cuh: -0.0 folded onto +0.0, NaN counted
+// and left out).  A 4 x 8-bit radix select over the impostor keys finds the (k+1)-th largest for up to 8 FARs at once:
+// per pass, the unresolved selections with the same key prefix share one histogram (prefixes of one length are equal
+// or disjoint, so each key lands in at most one), counted with warp-aggregated shared atomics; the last block to finish
+// a pass picks the bins.  One counting pass then accepts score > threshold for every FAR.  No sort of the scores.
 //
 // ROC curve (sklearn.metrics.roc_curve with drop_intermediate): the TAR keys, complemented so that ascending order is
 // descending score, are sorted with a stable 4 x 8-bit LSD radix sort that carries the class byte (per pass: a tile
@@ -35,6 +35,7 @@
 // fixed-order sums: the result does not depend on the schedule.
 #include "common.cuh"
 #include "../../fedfr_b200/csrc/dot_chain.cuh"
+#include "../../fedfr_b200/csrc/score_key.cuh"
 
 namespace pfc {
 
@@ -151,14 +152,6 @@ struct TarState {
   unsigned long long n_gen, n_imp, n_nan;
   unsigned long long acc_gen[kTarMaxFar], acc_imp[kTarMaxFar];
 };
-
-// Order-preserving key of an fp32 score given as its bits: larger score -> larger key; -0.0 and +0.0 -> one key.
-// NaN -> 0, which no number maps to (0 is the key of the bit pattern 0xffffffff, itself a NaN).
-__device__ __forceinline__ unsigned int tar_key(unsigned int u) {
-  if ((u & 0x7fffffffu) > 0x7f800000u) return 0u;
-  if ((u & 0x7fffffffu) == 0u) u = 0u;
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
 
 __global__ void tar_init_kernel(TarState* st) {
   unsigned int* h = &st->hist[0][0];

@@ -7,9 +7,12 @@
     fpr, tpr, thresholds = roc_curve(scores, issame)            # sklearn.metrics.roc_curve, element for element
     for far_target, tar, far in tar_at_far_nearest(fpr, tpr): ...   # the insightface IJB scripts' TAR table
     acc, best_thr, tpr, fpr = kfold_accuracy(emb, issame, flipped)  # the per-round LFW / CFP-FP / AgeDB K-fold test
+    rank, mate_score, top1_row, top1_score = mate_ranks(probe_feats, probe_subjects, gallery_feats, gallery_subjects)
+    cmc(rank, max_rank=20)                                          # 1:N identification: rank-1 ... rank-20 rates
+    for fpir_target, tpir, fpir, threshold in tpir_at_fpir(rank, mate_score, top1_score): ...
 
-The arithmetic is this repository's definition, pinned step by step (``include/fedfr_b200.h``, ``csrc/verify.cu``) so that
-a plain C restatement reproduces every feature and score bit for bit; it follows the usual insightface recipe (media
+The arithmetic is this repository's definition, pinned step by step (``include/fedfr_b200.h``, ``csrc/verify.cu``,
+``csrc/identify.cu``) so that a plain C restatement reproduces every feature and score bit for bit; it follows the usual insightface recipe (media
 mean, template sum, L2 normalise, cosine).  Inputs are CUDA tensors or numpy arrays; nothing runs on the CPU except
 index plumbing on the device (sorting ids into a CSR, id -> row lookup) and the final division of two counts.
 """
@@ -279,3 +282,100 @@ def kfold_accuracy(embeddings, issame, flipped=None, nfolds=10, thresholds=None)
                                          N.ptr(dist), N.ptr(acc), N.ptr(best), N.ptr(tpr), N.ptr(fpr), N.ptr(ws),
                                          ws.numel(), _stream(device)), "pfc_kfold_accuracy")
     return acc, best, tpr, fpr
+
+
+def mate_rows(probe_subjects, gallery_subjects):
+    """Gallery row of each probe's subject, -1 when the subject is not in the gallery, by a sort and a binary search on
+    the device.  ValueError when a subject occurs twice in the gallery (1:N here takes one entry per subject)."""
+    g_sorted, g_order = torch.sort(gallery_subjects)
+    if bool((g_sorted[1:] == g_sorted[:-1]).any()):
+        dup = int(g_sorted[1:][g_sorted[1:] == g_sorted[:-1]][0])
+        raise ValueError("gallery subject %d occurs more than once: the gallery needs one entry per subject" % dup)
+    r = torch.searchsorted(g_sorted, probe_subjects).clamp_(max=g_sorted.numel() - 1)
+    return torch.where(g_sorted[r] == probe_subjects, g_order[r], torch.full_like(r, -1))
+
+
+def mate_ranks(probe_feats, probe_subjects, gallery_feats, gallery_subjects):
+    """1:N identification (the IJB-B / IJB-C search protocol): for every probe, the rank of its mate in the gallery and
+    the gallery's top-1 match, exact, without a [P, G] score matrix.
+
+    probe_feats fp32 [P, E], gallery_feats fp32 [G, E] (used as given: normally ``template_features`` output);
+    probe_subjects int64 [P], gallery_subjects int64 [G] (one gallery entry per subject); CUDA tensors or numpy arrays.
+    A probe is mated when its subject is in the gallery.  Every score is the ``pair_scores`` chain, so it equals
+    ``pair_scores`` on the same two rows bit for bit.  rank = the mate's 1-based position in
+    ``np.argsort(-scores, kind="stable")`` (gallery order breaks ties; -0.0 == +0.0), 0 for a non-mated probe;
+    mate_score = its score (NaN when non-mated); top1_row / top1_score = the first gallery row with the largest score
+    and that score.  The definition is in ``include/fedfr_b200.h``.  Raises ValueError for duplicate gallery subjects
+    and for NaN scores (the check reads two counts back, which waits for the device).
+
+    IJB-C, once per gallery (G1, G2), with subjects from the protocol's template -> subject table::
+
+        feats_t, ids_t = template_features(img_feats, templates, medias, faceness)
+        probe_rows = torch.searchsorted(ids_t, probe_template_ids)     # the G1 / G2 template ids likewise
+        rank, mate_score, top1_row, top1_score = mate_ranks(feats_t[probe_rows], probe_subjects,
+                                                            feats_t[g1_rows], g1_subjects)
+        rank1 = cmc(rank, 1)[0]; tpir_fpir = tpir_at_fpir(rank, mate_score, top1_score)
+
+    -> (rank int64 [P], mate_score fp32 [P], top1_row int64 [P], top1_score fp32 [P]), CUDA tensors."""
+    device = _device(probe_feats)
+    x = _on(probe_feats, torch.float32, device)
+    y = _on(gallery_feats, torch.float32, device)
+    ps = _on(probe_subjects, torch.int64, device).reshape(-1)
+    gs = _on(gallery_subjects, torch.int64, device).reshape(-1)
+    if x.dim() != 2 or y.dim() != 2 or x.shape[0] == 0 or y.shape[0] == 0 or x.shape[1] == 0 or x.shape[1] != y.shape[1]:
+        raise ValueError("probe_feats [P, E] and gallery_feats [G, E] must be non-empty with one E")
+    if ps.numel() != x.shape[0] or gs.numel() != y.shape[0]:
+        raise ValueError("one subject per probe row and per gallery row")
+    m = mate_rows(ps, gs)
+    P = x.shape[0]
+    rank, top1_row, counts = (torch.empty(n, dtype=torch.int64, device=device) for n in (P, P, 2))
+    mate_score, top1_score = (torch.empty(P, dtype=torch.float32, device=device) for _ in range(2))
+    ws = torch.empty(int(N.lib.pfc_identify_workspace_bytes(P)), dtype=torch.uint8, device=device)
+    with torch.cuda.device(device):
+        N.check(N.lib.pfc_identify(N.ptr(x), P, N.ptr(y), y.shape[0], x.shape[1], N.ptr(m), N.ptr(rank),
+                                   N.ptr(mate_score), N.ptr(top1_row), N.ptr(top1_score), N.ptr(counts), N.ptr(ws),
+                                   ws.numel(), _stream(device)), "pfc_identify")
+    n_nan = int(counts[0])
+    if n_nan:
+        raise ValueError("%d probe-gallery scores are NaN" % n_nan)
+    return rank, mate_score, top1_row, top1_score
+
+
+def cmc(rank, max_rank=20):
+    """Cumulative match characteristic from ``mate_ranks``' ranks: cmc[r-1] = #{mated probes with rank <= r} / n_mated
+    for r = 1 ... max_rank (non-mated probes, rank 0, are left out).  ValueError without a mated probe.
+    -> float64 [max_rank] on the ranks' device."""
+    r = torch.as_tensor(rank).reshape(-1)
+    max_rank = int(max_rank)
+    if max_rank < 1:
+        raise ValueError("max_rank must be >= 1")
+    mated = r > 0
+    n_mated = int(mated.sum())
+    if n_mated == 0:
+        raise ValueError("cmc needs mated probes (got none)")
+    hits = torch.bincount(torch.where(mated, r.clamp(max=max_rank + 1), 0), minlength=max_rank + 2)[1:max_rank + 1]
+    hits = hits.cumsum(0).to(torch.float64)
+    return hits / torch.full_like(hits, n_mated)        # an IEEE division each (CUDA divides by a scalar as a product)
+
+
+def tpir_at_fpir(rank, mate_score, top1_score, fpirs=(1e-2, 1e-1), max_rank=1):
+    """TPIR at each target FPIR, at rank ``max_rank``, from ``mate_ranks``' outputs.  A non-mated probe's score is its
+    top-1 score; a mated probe's is its mate's score when rank <= max_rank, else -inf.  The result is exactly
+    ``tar_at_far`` of those scores with mated = genuine: the threshold is the (k+1)-th largest non-mated top-1 score,
+    k = floor(f * n_nonmated), and a mated probe counts iff its mate is within rank ``max_rank`` and scores above it.
+    ValueError without a mated or without a non-mated probe.  -> [(fpir_target, tpir, fpir, threshold)]."""
+    r = torch.as_tensor(rank).reshape(-1)
+    if int(max_rank) < 1:
+        raise ValueError("max_rank must be >= 1")
+    if not r.numel() == _numel(mate_score) == _numel(top1_score):
+        raise ValueError("rank, mate_score and top1_score need one entry per probe")
+    n_mated = int((r > 0).sum())
+    if n_mated == 0 or n_mated == r.numel():
+        raise ValueError("tpir_at_fpir needs mated and non-mated probes (got %d and %d)" % (n_mated, r.numel() - n_mated))
+    device = r.device if r.is_cuda else _device(mate_score)
+    r = r.to(device)
+    ms = _on(mate_score, torch.float32, device).reshape(-1)
+    ts = _on(top1_score, torch.float32, device).reshape(-1)
+    mated = r > 0
+    s = torch.where(mated, torch.where(r <= int(max_rank), ms, torch.full_like(ms, float("-inf"))), ts)
+    return tar_at_far(s, mated, fpirs)

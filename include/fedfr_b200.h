@@ -398,6 +398,34 @@ int pfc_kfold_accuracy(const float* emb, const float* flip, const unsigned char*
                        const double* thr, int n_thresholds, int64_t nfolds, float* dist, double* accuracy, double* best_thr,
                        double* tpr, double* fpr, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * 1:N identification (IJB-B / IJB-C search protocol)         ijbc_all.py rank-k, local_1n.py
+ * ------------------------------------------------------------------------------------------------
+ * probe fp32 [P, emb], gallery fp32 [G, emb] (used as given; normally pfc_template_pool output, one gallery row per
+ * subject), mate_row int64 [P]: the gallery row of the probe's subject, or -1 for a non-mated probe.  Gallery rows keep
+ * the caller's order, and that order breaks ties.
+ *   1. s(p, g) = (float)(sum_k (double)fl32(x_pk * y_gk)), k ascending: the pfc_pair_scores chain, so a pair's score
+ *      is bit-identical to pfc_pair_scores on the same two rows;
+ *   2. key(s) = the order-preserving uint32 key of pfc_tar_at_far: -0.0 folded onto +0.0; NaN maps to 0, below every
+ *      number, and is counted in n_nan;
+ *   3. mated probe with mate m: rank[p] = 1 + #{g : key_g > key_m} + #{g < m : key_g == key_m}, the mate's 1-based
+ *      position in np.argsort(-s_p, kind="stable"); rank[p] = 0 for a non-mated probe;
+ *      mate_score[p] = s(p, m), NaN without a mate;
+ *   4. top1_row[p] = the first row with the largest key (np.argsort(-s_p, kind="stable")[0]); top1_score[p] = its
+ *      score, read back from the key (so +0.0 for a zero score; NaN only when every score of the row is NaN).
+ * CMC and TPIR@FPIR follow from rank, mate_score and top1_score alone (fedfr_b200.verify cmc / tpir_at_fpir):
+ *   cmc[r-1] = #{mated p : rank_p <= r} / n_mated;  TPIR@FPIR at rank R is pfc_tar_at_far over s'_p = mate_score_p if
+ *   1 <= rank_p <= R else -inf (mated, "genuine") and s'_p = top1_score_p (non-mated, "impostor").
+ * A mate_row outside [-1, G) gets rank 0 and a NaN mate_score, like a bad row in pfc_pair_scores, and is counted.
+ * Writes rank, top1_row int64 [P], mate_score, top1_score fp32 [P] and counts int64 [2] = {n_nan (NaN scores over
+ * all P x G pairs), n_bad (mate rows outside [-1, G))}.  Limits: 1 <= emb <= 4096, 1 <= P, G < 2^31.  Deterministic:
+ * integer atomics and a 64-bit maximum, no float atomics, no [P, G] matrix; the host is never synchronised.
+ * workspace: pfc_identify_workspace_bytes(P) bytes (about 12 P), 8-byte aligned. */
+size_t pfc_identify_workspace_bytes(int64_t n_probe);
+int pfc_identify(const float* probe, int64_t n_probe, const float* gallery, int64_t n_gallery, int emb,
+                 const int64_t* mate_row, int64_t* rank, float* mate_score, int64_t* top1_row, float* top1_score,
+                 int64_t* counts, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
